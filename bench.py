@@ -71,7 +71,14 @@ def parse_args():
     ap.add_argument("--no-uncut-statevector", dest="uncut_statevector", action="store_false")
     ap.add_argument("--profile", action="store_true",
                     help="timed region only (for runs under ncu): no e2e leg, no oracle report, no CPU baseline")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps of each workload, write what its last step computed to "
+                         "DIR/<workload>.<array>.npy (float64; a result of more than 2^21 entries as a fixed, "
+                         "seeded sample of its entries, their indices in <workload>.values_index.npy)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's results: it needs --impl ours")
+    return args
 
 
 def metric_name(workload: str, accuracy: float = 0.0) -> str:
@@ -323,8 +330,6 @@ def reference_arm(args) -> None:
         t, sample, cores, _ = cpu_reference_step(workload, args.seed, args.cpu_sample_bits, window=7 * i + 1, ctx=ctx)
         if i >= args.warmup:
             times.append(t)
-        if sum(times) > 240:
-            break
     if ctx.get("pool") is not None:
         ctx["pool"].close()
     val = statistics.mean(times)
@@ -462,6 +467,44 @@ def sim_work(virt, frags, device, fold: bool = True) -> dict:
             "instances": inst_total, "instances_simulated": runs, "passes_executed": passes}
 
 
+DUMP_MAX_ENTRIES = 1 << 21      # per workload: 16 MiB of values + 16 MiB of indices; the default run dumps < 64 MiB
+
+
+def dump_outputs(dirpath: str, workload: str, accuracy: float, res, n_out: int, K: int, rank: int,
+                 world: int) -> list:
+    """Write the DenseResult of the resident step's last step - what ``run_virtual_circuit_dense`` hands its
+    caller - as float64 .npy files: ``values`` (the full-circuit distribution) and ``stats`` ([total, minimum]
+    of the knitted quasi-distribution).  A distribution of more than DUMP_MAX_ENTRIES entries is sampled at
+    fixed indices (seed 0, drawn over the whole output, independent of the number of GPUs), written to
+    ``values_index``, so that two builds or two runs can be compared entry for entry.  A rank that holds a
+    slice of the output (no virtual gate, several GPUs) writes the sampled entries of its slice under names
+    ending in ``.rank<r>``; with virtual gates every rank holds the whole result and rank 0 writes it."""
+    import numpy as np
+    import torch
+    if K > 0 and rank != 0:
+        return []
+    os.makedirs(dirpath, exist_ok=True)
+    stem = workload.replace(":", "_") + (f"_acc{accuracy:g}" if accuracy else "")
+    suffix = f".rank{rank}" if world > 1 and K == 0 else ""
+    values, y0 = res.values, res.y_begin
+    arrays = {}
+    if (1 << n_out) <= DUMP_MAX_ENTRIES:
+        arrays["values"] = values.cpu().numpy()
+    else:
+        idx = np.sort(np.random.default_rng(0).choice(1 << n_out, size=DUMP_MAX_ENTRIES, replace=False))
+        idx = idx[(idx >= y0) & (idx < y0 + values.numel())]
+        local = torch.from_numpy(idx - y0).to(values.device)
+        arrays["values"] = values[local].cpu().numpy()
+        arrays["values_index"] = idx.astype(np.float64)             # exact: indices < 2^53
+    arrays["stats"] = np.array([res.total, res.minimum], dtype=np.float64)
+    names = []
+    for key, arr in arrays.items():
+        name = f"{stem}.{key}{suffix}.npy"
+        np.save(os.path.join(dirpath, name), np.ascontiguousarray(arr, dtype=np.float64))
+        names.append(name)
+    return names
+
+
 def measure(workload: str, args, env: dict, primary: bool, accuracy: float = 0.0, cpu: bool = False) -> dict:
     """Everything bench.py reports for one workload (one JSON object)."""
     import numpy as np
@@ -552,6 +595,8 @@ def measure(workload: str, args, env: dict, primary: bool, accuracy: float = 0.0
     launches = launches_per_step * steps
     ms_per_step = reduce_max(e0.elapsed_time(e1)) / steps
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
+    dumped = (dump_outputs(args.dump_outputs, workload, accuracy, rs.result(), n_out, K, rank, world)
+              if args.dump_outputs else None)
     # the three phases of the step, each on its own (graph replays, or eager launches under --no-graph)
     phases = rs.capture(phases=True) if use_graph else None
     stage("phase capture")
@@ -719,6 +764,8 @@ def measure(workload: str, args, env: dict, primary: bool, accuracy: float = 0.0
     }
     if K == 0:
         line["hbm_gbs"] = roofline["achieved"]
+    if dumped is not None:
+        line["dumped_outputs"] = {"dir": os.path.abspath(args.dump_outputs), "files": dumped}
     line.update(extra)
     barrier()                                         # nothing of this workload is in flight when its graphs,
     del rs, out                                       # buffers and executors go away
@@ -728,7 +775,8 @@ def measure(workload: str, args, env: dict, primary: bool, accuracy: float = 0.0
 def compact(line: dict) -> dict:
     """The figures of a secondary workload that go under other_workloads."""
     keep = ("value", "ms_per_step", "steps", "gpu_launches", "result_sum", "result_min", "oracle",
-            "fidelity_cut_vs_uncut", "fidelity_delta_vs_oracle", "max_abs_err_cut_vs_uncut_gpu", "cpu_baseline")
+            "fidelity_cut_vs_uncut", "fidelity_delta_vs_oracle", "max_abs_err_cut_vs_uncut_gpu", "cpu_baseline",
+            "dumped_outputs")
     out = {k: line[k] for k in keep if k in line and line[k] is not None}
     out["config"] = {k: line["config"][k] for k in ("fragments", "virtual_gates", "global_labels", "partition", "accuracy")}
     if line.get("e2e"):

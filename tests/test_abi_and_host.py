@@ -2,6 +2,8 @@
 import ctypes
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -37,15 +39,26 @@ def test_struct_layouts_match_header():
     assert ctypes.sizeof(_lib.QckSimPlan) == 8 + 24 + 4 + 64 + 4 + 160 + 16
 
 
+_NO_GPU_CHILD = f"""
+import pytest, torch
+from importlib import import_module
+assert not torch.cuda.is_available()
+with pytest.raises(RuntimeError):
+    import_module("{PKG}._lib").Handle(0)
+qd = import_module("{PKG}.quasi_distr")
+with pytest.raises(RuntimeError, match="no CPU fallback"):
+    qd.QuasiDistr({{0: 1.0}})
+print("NO_GPU_LOUD_FAILURE_OK")
+"""
+
+
 def test_no_gpu_means_loud_failure():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    with pytest.raises(RuntimeError):
-        _lib.Handle(0)
-    qd = import_module(f"{PKG}.quasi_distr")
-    with pytest.raises(RuntimeError, match="no CPU fallback"):
-        qd.QuasiDistr({0: 1.0})
+    """Without a device every entry point raises.  Checked in a child process that sees no device
+    (CUDA_VISIBLE_DEVICES empty), so that it runs on a machine with a GPU as well."""
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    res = subprocess.run([sys.executable, "-c", _NO_GPU_CHILD], cwd=ROOT, env=env, capture_output=True,
+                         text=True, timeout=600)
+    assert res.returncode == 0 and "NO_GPU_LOUD_FAILURE_OK" in res.stdout, res.stdout[-2000:] + res.stderr[-2000:]
 
 
 def test_generators_shapes_and_seed():

@@ -1,8 +1,7 @@
-"""circuit_from_qiskit against duck-typed fakes and the reference's real Virtual* classes (CPU)."""
+"""circuit_from_qiskit against duck-typed fakes, checked with the reference's stored tables (CPU)."""
 import numpy as np
 import pytest
 
-from oracle import ref_loader as rl
 from oracle import statevector as sv
 
 PKG = "hardwareawareoptimalquantumcircuitcuttingandknitting_b200"
@@ -90,21 +89,30 @@ def test_unknown_gate_needs_matrix_or_fails():
     assert np.array_equal(ours.data[0].operation.to_matrix(), np.array([[0, 1], [1, 0]]))
 
 
-@pytest.mark.skipif(not rl.available(), reason="reference tree not present (GPU box)")
-def test_reference_virtual_gate_objects_convert():
-    """The reference's REAL Virtual* instances (loaded under the qiskit stub) map to ours with the
-    same tables, including VirtualCPhase whose parameter was rewritten in place."""
-    vg, _ = rl.load()
-    for kind, theta in [("move", None), ("cx", None), ("cz", None), ("cy", None), ("rzz", 0.83), ("cp", 0.83)]:
-        ref_gate = rl.make_vgate(vg, kind, theta)
+def _reference_shaped_vgate(kind, theta, params_after_init):
+    """A stand-in for the reference's Virtual* instance of ``kind``: a barrier named after its class that
+    keeps the replaced gate as ``_original_gate`` and shares that gate's parameter list as ``_params``
+    (the list VirtualCPhase rewrites in place, to ``params_after_init``)."""
+    cls_name = {v: k for k, v in adapters.VIRTUAL_CLASS_KINDS.items()}[kind]
+    orig = FOp("swap", 2, [], label="wc") if kind == "move" else FOp(kind, 2, [] if theta is None else [theta])
+    gate = type(cls_name, (FOp,), {})("barrier", 2, [], f"{kind} cut")
+    gate._original_gate, gate._params = orig, orig.params
+    if params_after_init is not None:
+        orig.params[:] = params_after_init
+    return gate
+
+
+def test_reference_shaped_virtual_gates_convert(golden):
+    """Virtual* instances shaped like the reference's map to ours with the reference's own instantiation
+    tables (tests/golden/instantiation_tables.json), including VirtualCPhase whose parameter the reference
+    rewrites in place to -theta/2."""
+    for entry in golden("instantiation_tables.json"):
+        ref_gate = _reference_shaped_vgate(entry["kind"], entry["theta"], entry.get("params_after_init"))
         q, c = FReg(2, "frag0"), FReg(1, "c")
         qc = FCircuit([q], [c])
         qc.data.append(FIns(ref_gate, [q[0], q[1]]))
-        # the stub's Barrier does not define .name; qiskit's does ("barrier")
-        ref_gate.name = getattr(ref_gate, "_name", "barrier")
         ours = adapters.circuit_from_qiskit(qc).data[0].operation
         assert type(ours).__name__ == type(ref_gate).__name__
-        ref_table = rl.dump_table(ref_gate)
         got = [[[i.operation.name, inst.qubits.index(i.qubits[0]), len(i.clbits), list(i.operation.params)]
                 for i in inst.data] for inst in ours._instantiations()]
-        assert got == ref_table, kind
+        assert got == entry["table"], (entry["kind"], entry["theta"])

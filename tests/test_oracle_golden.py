@@ -13,7 +13,6 @@ import pytest
 from conftest import load_golden, make_semcheck_circuit, oracle_knit
 from oracle import dense as od
 from oracle import qpd_tables as qt
-from oracle import ref_loader as rl
 from oracle import sparse_knit as sk
 
 PKG = "hardwareawareoptimalquantumcircuitcuttingandknitting_b200"
@@ -179,16 +178,7 @@ def test_hellinger_identities():
     assert abs(od.hellinger_fidelity_dense(a, b) - bc ** 2) < 1e-15
 
 
-# --------------------------------------------------------------------- (6) live re-check when the reference is here
-@pytest.mark.skipif(not rl.available(), reason="reference tree not present (GPU box)")
-def test_live_reference_agrees_with_fixture():
-    vg, qd = rl.load()
-    for entry in load_golden("instantiation_tables.json"):
-        g = rl.make_vgate(vg, entry["kind"], entry["theta"])
-        assert rl.dump_table(g) == entry["table"]
-
-
-# --------------------------------------------------------------------- (7) dense closed form == sparse driver
+# --------------------------------------------------------------------- (6) dense closed form == sparse driver
 def test_dense_contract_equals_sparse_driver():
     from oracle import statevector as sv
     for gname, theta in [("cx", None), ("rzz", 0.83)]:
