@@ -18,6 +18,7 @@ __all__ = [
     "VirtualGateEndpoint", "VirtualMove", "VirtualRZZ", "WireCut",
     "VirtualCircuit", "QuasiDistr", "run_virtual_circuit", "run_virtual_circuit_dense", "RunTimeInfo",
     "B200Backend", "hellinger_fidelity", "ResidentStep",
+    "expectation_values", "bitstring_probabilities", "marginal_distribution",
 ]
 
 _LAZY = {
@@ -29,6 +30,9 @@ _LAZY = {
     "B200Backend": ("backend", "B200Backend"),
     "hellinger_fidelity": ("fidelity", "hellinger_fidelity"),
     "ResidentStep": ("resident", "ResidentStep"),
+    "expectation_values": ("observables", "expectation_values"),
+    "bitstring_probabilities": ("observables", "bitstring_probabilities"),
+    "marginal_distribution": ("observables", "marginal_distribution"),
 }
 
 

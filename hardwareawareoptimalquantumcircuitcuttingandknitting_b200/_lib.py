@@ -135,6 +135,13 @@ _PROTOTYPES = {
                                          C.POINTER(C.c_int64), C.c_int, C.c_int, C.POINTER(QckFaithfulGate),
                                          C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_uint8), C.c_double,
                                          C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    "qck_rows_wht": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p, C.c_int64,
+                               C.c_void_p]),
+    "qck_rows_marginal": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_uint64, C.c_void_p,
+                                    C.c_void_p]),
+    "qck_knit_terms": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_int64), C.c_int,
+                                 C.POINTER(C.c_int32), C.POINTER(C.c_double), C.POINTER(C.c_int32), C.c_int64,
+                                 C.c_void_p, C.c_void_p, C.c_void_p]),
     "qck_stats_dense": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.c_void_p, C.c_void_p]),
     "qck_hellinger": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
     "qck_npd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.POINTER(C.c_double),

@@ -911,6 +911,29 @@ static unsigned long long compress_mask(unsigned long long mask, unsigned long l
 
 int qck_ensure_scratch(qck_handle* h, size_t bytes, void** out);  // api.cu
 
+// w[i] and rows[f][i] of the labels l_begin + i, i < count (also the label decode of qck_knit_terms, observe.cu)
+int qck_contract_prep(qck_handle* h, int n_frag, int n_digits, const int32_t* radix, const double* coef,
+                      const int32_t* frag_stride, long long l_begin, long long count, double* d_w, int* d_rows,
+                      cudaStream_t st) {
+    PrepParams pp;
+    memset(&pp, 0, sizeof(pp));
+    pp.n_digits = n_digits;
+    pp.n_frag = n_frag;
+    for (int k = 0; k < n_digits; ++k) {
+        pp.radix[k] = radix[k];
+        for (int v = 0; v < QCK_MAX_VARIANTS; ++v) pp.coef[k][v] = coef[k * QCK_MAX_VARIANTS + v];
+        for (int f = 0; f < n_frag; ++f) pp.stride[f][k] = frag_stride[f * QCK_MAX_DIGITS + k];
+    }
+    pp.l_begin = l_begin;
+    pp.count = count;
+    pp.w = d_w;
+    pp.rows = d_rows;
+    int pgrid = (int)((count + 255) / 256 < 1024 ? (count + 255) / 256 : 1024);
+    contract_prep_kernel<<<pgrid, 256, 0, st>>>(pp);
+    QCK_CHECK_LAUNCH(h);
+    return QCK_OK;
+}
+
 extern "C" int qck_knit_contract(qck_handle* h, int n_frag, const double* const* d_tables, const uint64_t* masks,
                                  const int64_t* row_strides, int n_out_bits, int n_digits, const int32_t* radix,
                                  const double* coef, const int32_t* frag_stride, int64_t l_begin, int64_t l_end,
@@ -1081,22 +1104,8 @@ extern "C" int qck_knit_contract(qck_handle* h, int n_frag, const double* const*
         }
     }
 
-    PrepParams pp;
-    memset(&pp, 0, sizeof(pp));
-    pp.n_digits = n_digits;
-    pp.n_frag = n_eff;
-    for (int k = 0; k < n_digits; ++k) {
-        pp.radix[k] = radix[k];
-        for (int v = 0; v < QCK_MAX_VARIANTS; ++v) pp.coef[k][v] = coef[k * QCK_MAX_VARIANTS + v];
-        for (int f = 0; f < n_eff; ++f) pp.stride[f][k] = fstr[f * QCK_MAX_DIGITS + k];
-    }
-    pp.l_begin = l_begin;
-    pp.count = count;
-    pp.w = d_w;
-    pp.rows = d_rows;
-    int pgrid = (int)((count + 255) / 256 < 1024 ? (count + 255) / 256 : 1024);
-    contract_prep_kernel<<<pgrid, 256, 0, st>>>(pp);
-    QCK_CHECK_LAUNCH(h);
+    rc = qck_contract_prep(h, n_eff, n_digits, radix, coef, fstr, l_begin, count, d_w, d_rows, st);
+    if (rc) return rc;
 
     ContractParams cp;
     memset(&cp, 0, sizeof(cp));

@@ -145,26 +145,32 @@ def run_virtual_circuit_dense(virt: VirtualCircuit, shots: int = 20000, device=N
         values = virt.knit_tables(tables, device, label_range=label_range, out=out)
         if label_range is not None:
             qdist.allreduce_sum_(values, group)
-        if nearest:
-            # statistics, threshold search and shift are all enqueued (qck_npd_async: no host round
-            # trip); the statistics of the knitted quasi-distribution come back with its state
-            ws = handle.npd_workspace(torch, device)
-            handle.check(handle.lib.qck_npd_async(handle.ptr, values.data_ptr(), values.numel(), 0.0,
-                                                  ws.data_ptr(), stream))
-            state = _check_npd_state(ws)          # the step's device -> host read (synchronises)
-            total, minimum = float(state[0]), float(state[1])
-        else:
-            stats = torch.zeros(4, dtype=torch.float64, device=device)
-            handle.check(handle.lib.qck_stats_dense(handle.ptr, values.data_ptr(), values.numel(), 0.0,
-                                                    stats.data_ptr(), stream))
-            host_stats = stats.cpu().numpy()
-            total, minimum = float(host_stats[0]), float(host_stats[1])
+        total, minimum = _finish_dense(handle, values, nearest, device, stream)
     ev[2].record()
     ev[2].synchronize()
     # device time of the two phases (run.py:60,67 take wall-clock times around the same two phases)
     run_time, knit_time = ev[0].elapsed_time(ev[1]) * 1e-3, ev[1].elapsed_time(ev[2]) * 1e-3
     logger.info(f"Knitted in {knit_time:.2f}s.")
     return DenseResult(values, union, total, minimum, y_begin), RunTimeInfo(run_time, knit_time)
+
+
+def _finish_dense(handle, values, nearest: bool, device, stream) -> tuple[float, float]:
+    """Total and minimum of a knitted dense quasi-distribution (synchronises); with ``nearest`` it is
+    then replaced in place by ``nearest_probability_distribution``."""
+    import torch
+    if nearest:
+        # statistics, threshold search and shift are all enqueued (qck_npd_async: no host round
+        # trip); the statistics of the knitted quasi-distribution come back with its state
+        ws = handle.npd_workspace(torch, device)
+        handle.check(handle.lib.qck_npd_async(handle.ptr, values.data_ptr(), values.numel(), 0.0,
+                                              ws.data_ptr(), stream))
+        state = _check_npd_state(ws)          # the step's device -> host read (synchronises)
+        return float(state[0]), float(state[1])
+    stats = torch.zeros(4, dtype=torch.float64, device=device)
+    handle.check(handle.lib.qck_stats_dense(handle.ptr, values.data_ptr(), values.numel(), 0.0,
+                                            stats.data_ptr(), stream))
+    host_stats = stats.cpu().numpy()
+    return float(host_stats[0]), float(host_stats[1])
 
 
 def _check_npd_state(ws, solved: bool = True):

@@ -358,15 +358,23 @@ class VirtualCircuit:
         return masks, union
 
     def knit_tables(self, tables: dict, device=None, label_range: tuple[int, int] | None = None,
-                    out=None, y_range: tuple[int, int] | None = None, stats=None, exchange=None):
+                    out=None, y_range: tuple[int, int] | None = None, stats=None, exchange=None,
+                    masks: dict | None = None):
         """Dense exact knit.  Returns a device tensor over the written clbits (index bit j = j-th
-        written clbit in ascending order; for ``measure_all`` circuits index == key)."""
+        written clbit in ascending order; for ``measure_all`` circuits index == key).  ``masks``:
+        {fragment: clbit mask of its table's columns} when the tables cover fewer clbits than the
+        fragments write (marginalised tables); the result then lives on the union of these masks."""
         import torch
         device = default_device() if device is None else device
         handle = _lib.get_handle(getattr(device, "index", None) or 0)
         stream = torch.cuda.current_stream(device).cuda_stream
         frags = list(tables.keys())
-        masks, union = self.output_masks(frags)
+        if masks is None:
+            masks, union = self.output_masks(frags)
+        else:
+            union = 0
+            for f in frags:
+                union |= masks[f]
         n_out = bin(union).count("1")
         cmask = [_compress_mask(masks[f], union) for f in frags]
         ptrs = (C.c_void_p * len(frags))(*[tables[f].data_ptr() for f in frags])
@@ -388,18 +396,7 @@ class VirtualCircuit:
             return out
         if y_range is not None:
             raise NotImplementedError("output sharding is only available without virtual gates")
-        self._check_limits(len(frags), K)
-        radices = self.global_radices()
-        coef = (C.c_double * (K * _lib.MAX_VARIANTS))()
-        for k, vg in enumerate(self.vgates):
-            for i, (a, _b) in enumerate(vg.knit_coefficients()):
-                coef[k * _lib.MAX_VARIANTS + i] = a       # signed fold already carries the -b half
-        strides = (C.c_int32 * (len(frags) * _lib.MAX_DIGITS))()
-        for i, f in enumerate(frags):
-            for k, s in enumerate(self._fragment_strides(f)):
-                strides[i * _lib.MAX_DIGITS + k] = s
-        row_strides = (C.c_int64 * len(frags))(*[tables[f].shape[1] for f in frags])
-        rad = (C.c_int32 * K)(*radices)
+        rad, coef, strides, row_strides = self._label_arrays(tables)
         l0, l1 = label_range if label_range is not None else (0, self.num_global_labels())
         if out is None:
             out = torch.empty(1 << n_out, dtype=torch.float64, device=device)
@@ -409,6 +406,24 @@ class VirtualCircuit:
             handle.check(handle.lib.qck_stats_dense(handle.ptr, out.data_ptr(), out.numel(), 0.0,
                                                     stats.data_ptr(), stream))
         return out
+
+    def _label_arrays(self, tables: dict) -> tuple:
+        """The label arrays of ``qck_knit_contract`` / ``qck_knit_terms`` for the fragments of ``tables``, in
+        its order: (radix [K], coef [K][QCK_MAX_VARIANTS], frag_stride [F][QCK_MAX_DIGITS], row strides [F])."""
+        frags = list(tables.keys())
+        K = len(self._vgate_instrs)
+        self._check_limits(len(frags), K)
+        coef = (C.c_double * (K * _lib.MAX_VARIANTS))()
+        for k, vg in enumerate(self.vgates):
+            for i, (a, _b) in enumerate(vg.knit_coefficients()):
+                coef[k * _lib.MAX_VARIANTS + i] = a       # signed fold already carries the -b half
+        strides = (C.c_int32 * (len(frags) * _lib.MAX_DIGITS))()
+        for i, f in enumerate(frags):
+            for k, s in enumerate(self._fragment_strides(f)):
+                strides[i * _lib.MAX_DIGITS + k] = s
+        row_strides = (C.c_int64 * len(frags))(*[tables[f].shape[1] for f in frags])
+        rad = (C.c_int32 * K)(*self.global_radices())
+        return rad, coef, strides, row_strides
 
     def _check_limits(self, n_frag: int, K: int) -> None:
         """The C ABI's fixed-size arrays (qck.h: QCK_MAX_FRAGMENTS, QCK_MAX_DIGITS, QCK_MAX_VARIANTS, int32

@@ -394,6 +394,29 @@ QCK_API int qck_knit_faithful_part(qck_handle* h, int n_frag, const double* cons
                                    const uint8_t* measures, double accuracy, double* d_out, int part, int n_parts,
                                    qck_stream stream);
 
+/* ------------------------------------------------------------------ observables from the fragment tables
+ * Expectation values, bitstring probabilities and marginals of the knitted (exact, unpruned) quasi-distribution
+ * without the dense 2^n_out vector (observables.py).  The knit is linear in every fragment table and the output
+ * masks are disjoint, so each quantity factorises over the fragments.  Fixed summation orders: deterministic.
+ * No host synchronisation; capturable in a CUDA graph once the handle's scratch holds what the call needs (an
+ * eager call of the same shape first).
+ *
+ * qck_rows_wht: out[r][s] = sum_x in[r][x] * (-1)^popcount(x & s) over 2^m_bits columns, for every row (out of
+ *   place; the unnormalised Walsh-Hadamard transform).  Then <Z_S> = sum_l w(l) prod_f W_f[lf(l)][pext(S, mask_f)].
+ * qck_rows_marginal: out[r][c] = sum_{x : pext(x, keep_mask) = c} in[r][x]; d_out is dense,
+ *   [n_rows][2^popcount(keep_mask)].
+ * qck_knit_terms: out[p] = sum_l w(l) prod_f T_f[lf(l)][cols[f][p]] over ALL global labels, w / lf / radix / coef /
+ *   frag_stride as for qck_knit_contract (n_digits = 0: one label of weight 1).  d_cols: DEVICE array
+ *   [n_frag][n_terms] of column indices (int64).  On Walsh-Hadamard rows it gives expectation values, on the
+ *   fragment tables themselves entries of the knitted distribution. */
+QCK_API int qck_rows_wht(qck_handle* h, const double* d_in, int64_t n_rows, int64_t row_stride, int m_bits,
+                         double* d_out, int64_t out_row_stride, qck_stream stream);
+QCK_API int qck_rows_marginal(qck_handle* h, const double* d_in, int64_t n_rows, int64_t row_stride, int m_bits,
+                              uint64_t keep_mask, double* d_out, qck_stream stream);
+QCK_API int qck_knit_terms(qck_handle* h, int n_frag, const double* const* d_tables, const int64_t* row_strides,
+                           int n_digits, const int32_t* radix, const double* coef, const int32_t* frag_stride,
+                           int64_t n_terms, const int64_t* d_cols, double* d_out, qck_stream stream);
+
 /* ------------------------------------------------------------------ reductions
  * qck_stats_dense: sum / min / nnz of a dense vector (entries |v| <= acc count as absent).
  * qck_hellinger: result[0..2] = sum p, sum q, sum sqrt(p q) over max(.,0) entries; the
