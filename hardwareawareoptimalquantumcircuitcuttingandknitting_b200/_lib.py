@@ -32,6 +32,7 @@ SWEEP_WARP = 8              # qck_sweep.flags: QCK_SWEEP_WARP (bits 8-15: fragme
 CLUSTER_QUBITS = 3
 NPD_STATS, NPD_PLAN, NPD_LEVEL, NPD_SELECT, NPD_APPLY = 0, 1, 2, 3, 4      # qck_npd_stage stages
 NPD_STATE_SLOTS, NPD_BINS, NPD_LEVEL_PASSES = 32, 8192, 6
+SAMPLE_ST_ENTRY, SAMPLE_ST_TOTAL = 1, 2   # qck_rows_sample status bits
 NPD_ST_SEARCH, NPD_ST_IDENTITY, NPD_ST_SOLVED, NPD_ST_NEGATIVE_TOTAL, NPD_ST_LOCATED = 0, 1, 2, 3, 4
 
 
@@ -142,6 +143,9 @@ _PROTOTYPES = {
     "qck_knit_terms": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_int64), C.c_int,
                                  C.POINTER(C.c_int32), C.POINTER(C.c_double), C.POINTER(C.c_int32), C.c_int64,
                                  C.c_void_p, C.c_void_p, C.c_void_p]),
+    "qck_rows_sample": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_int64, C.c_uint64,
+                                  C.c_uint32, C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p,
+                                  C.c_void_p]),
     "qck_stats_dense": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.c_void_p, C.c_void_p]),
     "qck_hellinger": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
     "qck_npd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.POINTER(C.c_double),

@@ -15,6 +15,10 @@ every fragment table and the fragments' output masks are disjoint, so each quant
 All of them work on the EXACT (unpruned) knitted quasi-distribution, as ``run_virtual_circuit_dense(...,
 nearest=False)`` returns it.  ``nearest_probability_distribution`` is not linear: the npd of a marginal is not the
 marginal of the npd, and an expectation value of the npd'd distribution needs that whole distribution.
+
+Finite-shot estimates take sampled tables unchanged: with every fragment on ``B200Backend(sampling=True, seed=s)``,
+``expectation_values(virt, z_masks, tables=virt.simulate_fragments(device, shots=N))`` is the estimate the reference's
+``shots``-sample run would give (the functions themselves take no ``shots``).
 """
 from __future__ import annotations
 

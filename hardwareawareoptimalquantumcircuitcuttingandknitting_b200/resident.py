@@ -29,6 +29,10 @@ class ResidentStep:
                  world_size: int = 1, group=None, accuracy: float = 0.0, out=None, graph: bool = True) -> None:
         import torch
         from . import dist as qdist
+        if virt.sampling_fragments():
+            # a replayed step would redraw the same seed: every replay would return the same sample
+            raise NotImplementedError("ResidentStep runs exact fragment tables; a fragment is bound to a "
+                                      "sampling B200Backend (use run_virtual_circuit_dense)")
         self.torch, self.qdist = torch, qdist
         self.virt = virt
         self.device = default_device() if device is None else torch.device(device)

@@ -4,10 +4,13 @@ Mirror of ``third_party/qvm/qvm/run.py:17-71`` with the reference signature
 ``run_virtual_circuit(virt, shots=20000) -> (dict[int, float], RunTimeInfo)``.
 
 When every fragment is bound to a ``B200Backend`` (the default) the whole path
-runs on the GPU from the compiled templates: exact outcome distributions instead
-of ``shots`` samples (``shots`` is accepted and ignored), signed-folded fragment
-tables, closed-form knit, ``nearest_probability_distribution`` on the dense
-vector.  ``run_virtual_circuit_dense`` is the same path returning the dense
+runs on the GPU from the compiled templates: signed-folded fragment tables,
+closed-form knit, ``nearest_probability_distribution`` on the dense vector.  With
+the default ``B200Backend()`` every instance contributes its exact outcome
+distribution and ``shots`` is ignored; with ``B200Backend(sampling=True, seed=s)``
+``shots`` is honoured as on Aer: every instance's distribution is sampled ``shots``
+times on the device (``VirtualCircuit.simulate_fragments(shots=)``) and the knit
+takes the sampled tables, so the result carries the reference's shot noise.  ``run_virtual_circuit_dense`` is the same path returning the dense
 device tensor - the only usable form at 32 output bits, where a Python dict of
 2^32 entries cannot exist.
 
@@ -103,8 +106,9 @@ def run_virtual_circuit_dense(virt: VirtualCircuit, shots: int = 20000, device=N
     K = len(virt._vgate_instrs)
     from . import quasi_distr as _qd
     accuracy = _qd.ACCURACY if accuracy is None else float(accuracy)
+    sample_shots = _sample_shots(virt, shots, world_size)
     if accuracy > 0.0:
-        return _run_faithful(virt, device, handle, nearest, accuracy, rank, world_size, group, out)
+        return _run_faithful(virt, device, handle, nearest, accuracy, rank, world_size, group, out, sample_shots)
     label_range = None
     if K > 0 and world_size > 1 and qdist.partition_mode(virt, world_size) == "label range + all-reduce":
         label_range = qdist.shard_range(virt.num_global_labels(), rank, world_size,
@@ -113,7 +117,8 @@ def run_virtual_circuit_dense(virt: VirtualCircuit, shots: int = 20000, device=N
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
     ev[0].record()
     logger.info(f"Running {sum(virt.program(f).num_labels for f in virt.active_fragments())} instances...")
-    tables = virt.simulate_fragments(device, label_range=label_range)
+    tables = virt.simulate_fragments(device, label_range=label_range, shots=sample_shots)
+    status = virt.sample_status if sample_shots is not None else None
     ev[1].record()
 
     logger.info("Knitting...")
@@ -131,7 +136,7 @@ def run_virtual_circuit_dense(virt: VirtualCircuit, shots: int = 20000, device=N
         values = virt.knit_tables(tables, device, stats=stats, y_range=y_range, out=out, exchange=ex)
         if ex is None:                            # (else the knit kernel's tail has exchanged them already)
             qdist.allreduce_stats(stats, group, handle)
-        host_stats = stats.cpu().numpy()          # the step's device -> host read (synchronises)
+        host_stats = _read_back(stats, status)    # the step's device -> host read (synchronises)
         total, minimum = float(host_stats[0]), float(host_stats[1])
         if nearest and minimum < 0.0:
             ws = handle.npd_workspace(torch, device)
@@ -145,7 +150,7 @@ def run_virtual_circuit_dense(virt: VirtualCircuit, shots: int = 20000, device=N
         values = virt.knit_tables(tables, device, label_range=label_range, out=out)
         if label_range is not None:
             qdist.allreduce_sum_(values, group)
-        total, minimum = _finish_dense(handle, values, nearest, device, stream)
+        total, minimum = _finish_dense(handle, values, nearest, device, stream, status)
     ev[2].record()
     ev[2].synchronize()
     # device time of the two phases (run.py:60,67 take wall-clock times around the same two phases)
@@ -154,9 +159,33 @@ def run_virtual_circuit_dense(virt: VirtualCircuit, shots: int = 20000, device=N
     return DenseResult(values, union, total, minimum, y_begin), RunTimeInfo(run_time, knit_time)
 
 
-def _finish_dense(handle, values, nearest: bool, device, stream) -> tuple[float, float]:
+def _sample_shots(virt: VirtualCircuit, shots: int, world_size: int) -> int | None:
+    """``shots`` when some fragment's backend samples, else None (exact tables)."""
+    sampling = virt.sampling_fragments()
+    if not sampling:
+        return None
+    if world_size > 1 and any(virt.get_backend(f).seed is None for f in sampling):
+        raise ValueError("a sampled multi-rank run needs B200Backend(sampling=True, seed=<int>): every rank must "
+                         "draw the same counts")
+    return int(shots)
+
+
+def _read_back(stats, status=None):
+    """stats (float64 device vector) -> host numpy; with the sampler's status word appended in the same copy
+    (raises when it is set)."""
+    import torch
+    if status is None:
+        return stats.cpu().numpy()
+    host = torch.cat([stats.view(torch.int64), status]).cpu()
+    from .sampling import raise_for_status
+    raise_for_status(int(host[-1]))
+    return host[:-1].view(torch.float64).numpy()
+
+
+def _finish_dense(handle, values, nearest: bool, device, stream, status=None) -> tuple[float, float]:
     """Total and minimum of a knitted dense quasi-distribution (synchronises); with ``nearest`` it is
-    then replaced in place by ``nearest_probability_distribution``."""
+    then replaced in place by ``nearest_probability_distribution``.  ``status``: the sampler's status word,
+    read back with the statistics."""
     import torch
     if nearest:
         # statistics, threshold search and shift are all enqueued (qck_npd_async: no host round
@@ -164,20 +193,27 @@ def _finish_dense(handle, values, nearest: bool, device, stream) -> tuple[float,
         ws = handle.npd_workspace(torch, device)
         handle.check(handle.lib.qck_npd_async(handle.ptr, values.data_ptr(), values.numel(), 0.0,
                                               ws.data_ptr(), stream))
-        state = _check_npd_state(ws)          # the step's device -> host read (synchronises)
+        state = _check_npd_state(ws, status=status)   # the step's device -> host read (synchronises)
         return float(state[0]), float(state[1])
     stats = torch.zeros(4, dtype=torch.float64, device=device)
     handle.check(handle.lib.qck_stats_dense(handle.ptr, values.data_ptr(), values.numel(), 0.0,
                                             stats.data_ptr(), stream))
-    host_stats = stats.cpu().numpy()
+    host_stats = _read_back(stats, status)
     return float(host_stats[0]), float(host_stats[1])
 
 
-def _check_npd_state(ws, solved: bool = True):
+def _check_npd_state(ws, solved: bool = True, status=None):
     """Reads the 256-byte state qck_npd_async / npd_sharded left in the workspace (synchronises) and
-    raises where the reference would fail (negative total: quasi_distr.py:36 ends in a division by zero)."""
+    raises where the reference would fail (negative total: quasi_distr.py:36 ends in a division by zero).
+    ``status``: the sampler's status word, read in the same copy."""
     import torch
-    state = ws[:_lib.NPD_STATE_SLOTS].cpu()
+    if status is not None:
+        host = torch.cat([ws[:_lib.NPD_STATE_SLOTS], status]).cpu()
+        from .sampling import raise_for_status
+        raise_for_status(int(host[-1]))
+        state = host[:-1]
+    else:
+        state = ws[:_lib.NPD_STATE_SLOTS].cpu()
     status = int(state[5])
     state = state.view(torch.float64).numpy()
     if solved and status == _lib.NPD_ST_NEGATIVE_TOTAL:
@@ -187,7 +223,7 @@ def _check_npd_state(ws, solved: bool = True):
     return state
 
 
-def _run_faithful(virt, device, handle, nearest, accuracy, rank, world_size, group, out):
+def _run_faithful(virt, device, handle, nearest, accuracy, rank, world_size, group, out, shots=None):
     """ACCURACY > 0: exact instance distributions, then the reference's pruned algebra in the
     reference's order, fused per output entry (``qck_knit_faithful``).  Every output entry is an
     independent expression tree: with ``world_size > 1`` every rank simulates the (small) fragments itself,
@@ -197,7 +233,8 @@ def _run_faithful(virt, device, handle, nearest, accuracy, rank, world_size, gro
     stream = torch.cuda.current_stream(device).cuda_stream
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
     ev[0].record()
-    tables = virt.simulate_fragments(device, fold=False)
+    tables = virt.simulate_fragments(device, fold=False, shots=shots)
+    status = virt.sample_status if shots is not None else None
     ev[1].record()
     logger.info("Knitting...")
     sharded = world_size > 1 and len(virt._vgate_instrs) > 0
@@ -211,7 +248,7 @@ def _run_faithful(virt, device, handle, nearest, accuracy, rank, world_size, gro
     else:
         handle.check(handle.lib.qck_npd_stage(handle.ptr, _lib.NPD_STATS, values.data_ptr(), values.numel(),
                                               accuracy, ws.data_ptr(), 1, stream))
-    state = _check_npd_state(ws, solved=nearest)
+    state = _check_npd_state(ws, solved=nearest, status=status)
     total, minimum = float(state[0]), float(state[1])
     ev[2].record()
     ev[2].synchronize()
@@ -308,6 +345,8 @@ def run_virtual_circuit(virt: VirtualCircuit, shots: int = 20000) -> tuple[dict[
     accuracy = float(_qd.ACCURACY)
     fold = accuracy <= 0.0
     jobs, tables = {}, {}
+    from .sampling import new_status
+    status = None
     frags = virt.fragment_circuits
     logger.info(f"Running virtualizer with {len(frags)} "
                 + f"{tuple(circ.num_qubits for circ in frags.values())} "
@@ -320,7 +359,13 @@ def run_virtual_circuit(virt: VirtualCircuit, shots: int = 20000) -> tuple[dict[
         num_instances += len(instance_labels)
         if isinstance(backend, B200Backend):
             if virt.program(frag).measures_anything:
-                tables[frag] = virt.executor(frag, device, fold).run(handle)
+                if backend.sampling:
+                    status = new_status(torch, device) if status is None else status
+                    unfolded = virt.executor(frag, device, False).run(handle)
+                    tables[frag] = virt.sample_table(handle, frag, unfolded, fold, shots, status,
+                                                     stream=torch.cuda.current_stream(device).cuda_stream)
+                else:
+                    tables[frag] = virt.executor(frag, device, fold).run(handle)
             continue
         instantiations = generate_instantiations(frag_circuit, instance_labels)
         jobs[frag] = (backend.run(instantiations, shots=shots), len(instantiations))
@@ -343,7 +388,7 @@ def run_virtual_circuit(virt: VirtualCircuit, shots: int = 20000) -> tuple[dict[
     ws = handle.npd_workspace(torch, device)
     handle.check(handle.lib.qck_npd_async(handle.ptr, values.data_ptr(), values.numel(), accuracy, ws.data_ptr(),
                                           stream))
-    state = _check_npd_state(ws)
+    state = _check_npd_state(ws, status=status)
     knit_time = perf_counter() - now
     logger.info(f"Knitted in {knit_time:.2f}s.")
     _, union = virt.output_masks(list(tables))

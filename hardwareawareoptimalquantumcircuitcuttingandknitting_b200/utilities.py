@@ -4,7 +4,9 @@
 each on an ideal simulator and on ``backend``, in four threads, and returns the three Hellinger fidelities
 ``(input ideal vs backend, cut ideal vs backend, uncut ideal vs cut ideal)`` (``Utilities.py:154-226``).  Here the
 ideal simulator is ``B200Backend`` in place of ``AerSimulator()`` - exact distributions, ``nShots`` only scales
-the float "counts" - and ``backend`` may be any duck-typed backend (``.run(circuits, shots=)`` ->
+the float "counts"; ``ideal_backend=B200Backend(sampling=True, seed=s)`` samples the ideal runs ``nShots`` times as
+the reference's AerSimulator does, so all three fidelities carry shot noise - and ``backend`` may be any duck-typed
+backend (``.run(circuits, shots=)`` ->
 ``job.result().get_counts()``), e.g. the reference's fake noisy ones; ``backend=None`` uses a second
 ``B200Backend``, so the first two fidelities are 1.  The handles behind the device calls are thread-local
 (``_lib.get_handle``), which is what lets the reference's thread structure stay.
@@ -49,27 +51,30 @@ def _as_dict(dist) -> dict[int, float]:
     return dist.to_dict() if isinstance(dist, QuasiDistr) else dict(dist)
 
 
-def getCircResultFromBackend(circuit, backend, nShots: int):
+def getCircResultFromBackend(circuit, backend, nShots: int, ideal_backend=None):
     """-> (ideal, backend) distributions of an uncut circuit (``Utilities.py:39-69``)."""
     def task(be):
         return QuasiDistr.from_counts(be.run(circuit, shots=nShots).result().get_counts(), accuracy=0.0)
-    return _run_pair(task, B200Backend(), B200Backend() if backend is None else backend)
+    return _run_pair(task, B200Backend() if ideal_backend is None else ideal_backend,
+                     B200Backend() if backend is None else backend)
 
 
-def getVirtualCircResultFromBackend(cutCircuit, backend, nShots: int):
+def getVirtualCircResultFromBackend(cutCircuit, backend, nShots: int, ideal_backend=None):
     """-> (ideal, backend) distributions of a cut circuit through ``run_virtual_circuit``
     (``Utilities.py:74-103``): one ``VirtualCircuit`` per thread, every fragment bound to that thread's backend."""
     def task(be):
         virt = VirtualCircuit(cutCircuit.copy())
         virt.set_backend_for_all(be)
         return run_virtual_circuit(virt, shots=nShots)[0]
-    return _run_pair(task, B200Backend(), B200Backend() if backend is None else backend)
+    return _run_pair(task, B200Backend() if ideal_backend is None else ideal_backend,
+                     B200Backend() if backend is None else backend)
 
 
-def compareOriginalCircWithCutCirc(originalCirc, cutCirc, backend=None, nShots: int = 1000):
-    """-> (inputCircFidelity, cutCircFidelity, cutVsUncutFidelity) (``Utilities.py:154-226``)."""
+def compareOriginalCircWithCutCirc(originalCirc, cutCirc, backend=None, nShots: int = 1000, ideal_backend=None):
+    """-> (inputCircFidelity, cutCircFidelity, cutVsUncutFidelity) (``Utilities.py:154-226``).  ``ideal_backend``:
+    the backend of the two ideal runs (default ``B200Backend()``, exact)."""
     (input_ideal, input_noisy), (cut_ideal, cut_noisy) = _run_pair(
-        lambda job: job[0](job[1], backend, nShots),
+        lambda job: job[0](job[1], backend, nShots, ideal_backend),
         (getCircResultFromBackend, originalCirc), (getVirtualCircResultFromBackend, cutCirc))
     n_bits = len(originalCirc.clbits)
     input_ideal, input_noisy, cut_ideal, cut_noisy = (_as_dict(d) for d in (input_ideal, input_noisy, cut_ideal,

@@ -303,13 +303,30 @@ class VirtualCircuit:
                 acc *= radices[k]
         return strides
 
+    def sampling_fragments(self) -> list[Fragment]:
+        """Active fragments bound to a ``B200Backend(sampling=True)``."""
+        from .backend import B200Backend
+        return [f for f in self.active_fragments()
+                if isinstance(self._frag_to_backend[f], B200Backend) and self._frag_to_backend[f].sampling]
+
     def simulate_fragments(self, device=None, label_range: tuple[int, int] | None = None,
-                           fold: bool = True, out: dict | None = None) -> dict:
+                           fold: bool = True, out: dict | None = None, shots: int | None = None) -> dict:
         """All instances of all active fragments -> {fragment: device tensor [L_f, 2^m_f]}.
         ``label_range`` (global labels) restricts the work to what one rank needs.  ``fold=False``
         keeps the config bits as extra column bits (input of the reference-faithful knit).  ``out``: tables to
-        write into (a resident step reuses its buffers)."""
+        write into (a resident step reuses its buffers).
+
+        ``shots``: every fragment whose backend samples (``B200Backend(sampling=True)``) is simulated unfolded and
+        each instance's row is replaced by a multinomial sample of ``shots`` divided by ``shots``, in the layout
+        ``fold`` asks for (``qck_rows_sample``; stream id = the fragment's index in ``fragment_circuits``, row label
+        = the fragment label, so label ranges draw the rows of the full run).  Fragments on exact backends are
+        unchanged.  The status word of the sampler is left in ``self.sample_status`` (device int64, 0 = the tables
+        were valid); ``check_sample_status()`` reads it.  Observables take these tables unchanged
+        (``expectation_values(virt, z_masks, tables=virt.simulate_fragments(dev, shots=N))``)."""
         device = default_device() if device is None else device
+        sampled = set(self.sampling_fragments()) if shots is not None else set()
+        if sampled:
+            return self._simulate_sampled(device, label_range, fold, out, int(shots), sampled)
         handle = _lib.get_handle(getattr(device, "index", None) or 0)
         import torch
         stream = torch.cuda.current_stream(device).cuda_stream
@@ -344,6 +361,53 @@ class VirtualCircuit:
         for ex, table in runs:
             ex.finish(handle, table)
         return tables
+
+    def _simulate_sampled(self, device, label_range, fold, out, shots, sampled) -> dict:
+        import torch
+        from . import sampling as _sampling
+        exact = self.simulate_fragments(device, label_range, fold=False, shots=None)
+        handle = _lib.get_handle(getattr(device, "index", None) or 0)
+        stream = torch.cuda.current_stream(device).cuda_stream
+        self.sample_status = _sampling.new_status(torch, device)
+        tables = {}
+        for frag, table in exact.items():
+            if frag not in sampled:
+                if fold:        # an exact fragment keeps its folded table
+                    table = self.executor(frag, device, True).run(
+                        handle, out=out[frag] if out is not None else None,
+                        label_range=self.fragment_label_range(frag, *label_range)
+                        if label_range is not None and self._vgate_instrs else None)
+                tables[frag] = table
+                continue
+            tables[frag] = self.sample_table(handle, frag, table, fold, shots, self.sample_status, label_range,
+                                             out[frag] if out is not None else None, stream)
+        return tables
+
+    def sample_table(self, handle, frag: Fragment, unfolded, fold: bool, shots: int, status,
+                     label_range: tuple[int, int] | None = None, out=None, stream: int = 0):
+        """Sampled table of one fragment from its unfolded exact table (``qck_rows_sample``)."""
+        import torch
+        from . import sampling as _sampling
+        prog = self.program(frag)
+        seed = self._frag_to_backend[frag].next_seed()
+        stream_id = list(self._frag_circs).index(frag)
+        l0, l1 = (0, prog.num_labels)
+        if label_range is not None and self._vgate_instrs:
+            l0, l1 = self.fragment_label_range(frag, *label_range)
+        if out is None:
+            alloc = torch.zeros if (l0, l1) != (0, prog.num_labels) else torch.empty
+            out = alloc((prog.num_labels, prog.row_len(fold)), dtype=torch.float64, device=unfolded.device)
+        f = 0 if not fold else len(prog.radix)
+        _sampling.rows_sample(handle, unfolded, prog.row_bits + len(prog.radix), shots, seed, stream_id, status,
+                              l0, l1, out=out, fold_bits=f, stream=stream)
+        return out
+
+    def check_sample_status(self) -> None:
+        """Raises ValueError when the last sampled ``simulate_fragments`` met an invalid table (synchronises)."""
+        from . import sampling as _sampling
+        status = getattr(self, "sample_status", None)
+        if status is not None:
+            _sampling.raise_for_status(int(status.item()))
 
     def output_masks(self, fragments=None) -> tuple[dict, int]:
         """-> ({fragment: clbit mask of its output row}, union).  The dense result lives on the

@@ -417,6 +417,39 @@ QCK_API int qck_knit_terms(qck_handle* h, int n_frag, const double* const* d_tab
                            int n_digits, const int32_t* radix, const double* coef, const int32_t* frag_stride,
                            int64_t n_terms, const int64_t* d_cols, double* d_out, qck_stream stream);
 
+/* ------------------------------------------------------------------ finite-shot sampling
+ * Replaces: backend.run(instantiations, shots) on AerSimulator + QuasiDistr.from_counts (run.py:42,
+ * quasi_distr.py:13-20): every instance is sampled `shots` times instead of returning its exact distribution.
+ *
+ * qck_rows_sample draws, for every row r of an UNFOLDED fragment table (simulate_fragments(fold=False): a row is an
+ * instance's joint distribution over its written clbits and config bits, the config bits the top fold_bits column
+ * bits), a multinomial of `shots` over its 2^m_bits columns.  Definition (tests/sampling_reference.py restates it):
+ *   - sum tree: s_0[x] = v[x], s_{j+1}[i] = s_j[2i] + s_j[2i+1] (doubles, exactly this pairing);
+ *   - the root s_m[0] gets `shots`; node (j, i), j >= 1, with count c > 0 gives its left child B(c, p),
+ *     p = s_{j-1}[2i] / s_j[i], and its right child the rest; when c = 0, p = 0 or p = 1 there is no draw and no
+ *     random number is consumed.  The leaves' counts are the sample;
+ *   - B(c, p): ATen's sample_binomial - inversion when c * min(p, 1 - p) < 10, else BTRS (Hormann 1993); for
+ *     p > 1/2 it draws c - B(c, 1 - p) with 1 - p rounded to double;
+ *   - random numbers: Philox4x32-10, key = (seed mod 2^32, seed >> 32), counter of the t-th Philox call of node
+ *     (j, i) of row r = (i mod 2^32, (i >> 32) | j << 16, row_label_begin + r, stream_id << 20 | t).  Call t gives
+ *     two uniforms, from (w0, w1) then (w2, w3): x = w_lo | w_hi << 32, u = ((x >> 11) | 1) * 2^-53, which lies in
+ *     [2^-53, 1 - 2^-53].  So the counts depend on (seed, stream id, row label, row values) only: not on how rows
+ *     are split over calls, ranks or CTAs.  Copies of one instance are separate rows and draw independently.
+ * Outputs (either or both):
+ *   d_out [n_rows][out_row_stride]: fold_bits = 0: count[x] / shots; fold_bits = f: the signed fold
+ *     (sum_c (-1)^popcount(c) count[x | c << (m - f)]) / shots over 2^(m - f) columns, summed in integers - equal,
+ *     bit for bit, to folding the counts of the unfolded output.  Padding past the row is not touched.
+ *   d_shot_list [n_rows][shots]: the drawn column indices in ascending order (for single wide rows).
+ * Entries must be finite and >= 0 and a row total > 0: otherwise bit 0 (an entry) / bit 1 (a total) is OR-ed into
+ * *d_status (device); a row whose total is not > 0 gets no shots.  1 <= shots < 2^31, stream_id < 2^12, labels < 2^32.  Rows of
+ * <= 2^13 columns: one CTA per row; wider ones: one pass writes the 2^12-column tile sums into the handle's scratch,
+ * the descent reads only the tiles that received shots again.  No host synchronisation; capturable once the
+ * handle's scratch is sized. */
+QCK_API int qck_rows_sample(qck_handle* h, const double* d_in, int64_t n_rows, int64_t row_stride, int m_bits,
+                            int64_t shots, uint64_t seed, uint32_t stream_id, int64_t row_label_begin,
+                            double* d_out, int64_t out_row_stride, int fold_bits, int64_t* d_shot_list,
+                            uint64_t* d_status, qck_stream stream);
+
 /* ------------------------------------------------------------------ reductions
  * qck_stats_dense: sum / min / nnz of a dense vector (entries |v| <= acc count as absent).
  * qck_hellinger: result[0..2] = sum p, sum q, sum sqrt(p q) over max(.,0) entries; the
