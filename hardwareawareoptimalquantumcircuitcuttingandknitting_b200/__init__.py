@@ -19,6 +19,7 @@ __all__ = [
     "VirtualCircuit", "QuasiDistr", "run_virtual_circuit", "run_virtual_circuit_dense", "RunTimeInfo",
     "B200Backend", "hellinger_fidelity", "ResidentStep",
     "expectation_values", "bitstring_probabilities", "marginal_distribution",
+    "NoiseModel", "QuantumError", "ReadoutError", "depolarizing_error", "thermal_relaxation_error", "kraus_error",
 ]
 
 _LAZY = {
@@ -33,6 +34,8 @@ _LAZY = {
     "expectation_values": ("observables", "expectation_values"),
     "bitstring_probabilities": ("observables", "bitstring_probabilities"),
     "marginal_distribution": ("observables", "marginal_distribution"),
+    **{name: ("noise", name) for name in ("NoiseModel", "QuantumError", "ReadoutError", "depolarizing_error",
+                                          "thermal_relaxation_error", "kraus_error")},
 }
 
 

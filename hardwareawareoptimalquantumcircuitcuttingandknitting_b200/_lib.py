@@ -75,6 +75,22 @@ class QckFaithfulGate(C.Structure):
                 ("cos_half_sq", C.c_double), ("sin_half_sq", C.c_double)]
 
 
+DM_MAX_TILE_BITS, DM_MAX_QUBITS = 12, 20
+
+
+class QckDmSweep(C.Structure):
+    _fields_ = [("n_tile", C.c_int32), ("op_begin", C.c_int32), ("op_end", C.c_int32),
+                ("pos", C.c_int32 * DM_MAX_TILE_BITS)]
+
+
+class QckDmPlan(C.Structure):
+    _fields_ = [("n_qubits", C.c_int32), ("n_sweeps", C.c_int32), ("sweeps", C.POINTER(QckDmSweep)),
+                ("d_ops", C.c_void_p), ("d_mats", C.c_void_p), ("d_items", C.c_void_p),
+                ("item_begin", C.POINTER(C.c_int64)), ("n_labels", C.c_int64), ("d_ro_mask", C.c_void_p),
+                ("d_ro", C.c_void_p), ("n_cols", C.c_int32), ("fold_bits", C.c_int32),
+                ("qcol", C.c_int32 * DM_MAX_QUBITS), ("n_digits", C.c_int32), ("radix", C.c_int32 * MAX_DIGITS)]
+
+
 class QckStats(C.Structure):
     _fields_ = [("sum", C.c_double), ("min", C.c_double), ("sum_sqrt", C.c_double), ("nnz", C.c_double)]
 
@@ -146,6 +162,8 @@ _PROTOTYPES = {
     "qck_rows_sample": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_int64, C.c_uint64,
                                   C.c_uint32, C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p,
                                   C.c_void_p]),
+    "qck_sim_density": (C.c_int, [C.c_void_p, C.POINTER(QckDmPlan), C.c_int64, C.c_int64, C.c_void_p, C.c_int64,
+                                  C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "qck_stats_dense": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.c_void_p, C.c_void_p]),
     "qck_hellinger": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
     "qck_npd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.POINTER(C.c_double),

@@ -17,6 +17,11 @@ the drawn column indices (at most ``shots`` of them) come back to the host, neve
 an integer makes every call reproducible (Aer's ``seed_simulator``), ``None`` draws a fresh seed per call.  The same
 backend bound to fragments makes ``run_virtual_circuit(virt, shots)`` sample every fragment instance.
 
+``B200Backend(noise_model=nm)`` (``noise.py``) simulates every circuit's density matrix under the noise model
+(``density.py``, ``qck_sim_density``): ``run``, ``exact_distribution`` and ``sample_counts`` then give the exact noisy
+distribution, or with ``sampling=True`` a multinomial of it - what a noisy Aer backend returns.  Bound to fragments,
+it gives every fragment instance its noisy table.  ``noise_model=None`` is the noiseless state-vector path.
+
 ``run_virtual_circuit`` recognises this class and bypasses circuit objects,
 strings and dicts entirely (``VirtualCircuit.simulate_fragments``).
 """
@@ -54,10 +59,11 @@ class B200Job:
 class B200Backend:
     name = "b200_statevector"
 
-    def __init__(self, device=None, sampling: bool = False, seed: int | None = None) -> None:
+    def __init__(self, device=None, sampling: bool = False, seed: int | None = None, noise_model=None) -> None:
         self._device = device
         self.sampling = bool(sampling)
         self.seed = seed
+        self.noise_model = noise_model
 
     def next_seed(self) -> int:
         """The Philox key of one call: ``seed``, or a fresh one when it is None."""
@@ -80,6 +86,12 @@ class B200Backend:
         flat = QuantumCircuit(whole, *circuit.cregs)
         for ins in circuit.data:
             flat.append(ins.operation, [remap[q] for q in ins.qubits], ins.clbits)
+        if self.noise_model is not None:
+            from .density import DensityExecutor, DensityProgram
+            prog = DensityProgram(flat, whole, circuit.num_clbits, self.noise_model)
+            if not prog.measures_anything:
+                return prog, None, handle
+            return prog, DensityExecutor(prog, device).run(handle), handle
         prog = FragmentProgram(flat, whole, circuit.num_clbits)
         if not prog.measures_anything:
             return prog, None, handle

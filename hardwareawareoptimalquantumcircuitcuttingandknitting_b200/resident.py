@@ -33,6 +33,9 @@ class ResidentStep:
             # a replayed step would redraw the same seed: every replay would return the same sample
             raise NotImplementedError("ResidentStep runs exact fragment tables; a fragment is bound to a "
                                       "sampling B200Backend (use run_virtual_circuit_dense)")
+        if virt.noisy_fragments():
+            raise NotImplementedError("ResidentStep runs state-vector fragment programs; a fragment is bound to a "
+                                      "noisy B200Backend (use run_virtual_circuit or run_virtual_circuit_dense)")
         self.torch, self.qdist = torch, qdist
         self.virt = virt
         self.device = default_device() if device is None else torch.device(device)

@@ -5,13 +5,15 @@ each on an ideal simulator and on ``backend``, in four threads, and returns the 
 ``(input ideal vs backend, cut ideal vs backend, uncut ideal vs cut ideal)`` (``Utilities.py:154-226``).  Here the
 ideal simulator is ``B200Backend`` in place of ``AerSimulator()`` - exact distributions, ``nShots`` only scales
 the float "counts"; ``ideal_backend=B200Backend(sampling=True, seed=s)`` samples the ideal runs ``nShots`` times as
-the reference's AerSimulator does, so all three fidelities carry shot noise - and ``backend`` may be any duck-typed
-backend (``.run(circuits, shots=)`` ->
-``job.result().get_counts()``), e.g. the reference's fake noisy ones; ``backend=None`` uses a second
-``B200Backend``, so the first two fidelities are 1.  The handles behind the device calls are thread-local
-(``_lib.get_handle``), which is what lets the reference's thread structure stay.
+the reference's AerSimulator does, so all three fidelities carry shot noise.
 
-Noise models are out of scope (SURVEY section 2, row 5): nothing here simulates noise.
+``backend=B200Backend(noise_model=nm, sampling=True, seed=s)`` (``noise.py``) is the noisy half of the reference's
+experiment: the uncut circuit and every fragment instance are simulated as density matrices under ``nm`` and
+sampled ``nShots`` times, a multinomial of the noisy distribution as a noisy Aer backend draws it; with
+``sampling=False`` the noisy distributions are exact.  ``backend`` may also be any duck-typed backend
+(``.run(circuits, shots=)`` -> ``job.result().get_counts()``), e.g. the reference's fake noisy ones;
+``backend=None`` uses a second noiseless ``B200Backend``, so the first two fidelities are 1.  The handles behind the
+device calls are thread-local (``_lib.get_handle``), which is what lets the reference's thread structure stay.
 """
 from __future__ import annotations
 

@@ -103,9 +103,12 @@ class VirtualCircuit:
         if fragment not in self._frag_to_backend:
             raise ValueError("Fragment not found.")
         self._frag_to_backend[fragment] = backend
+        # the executor depends on the backend (state vector, or density matrix under its noise model)
+        self._executors = {k: v for k, v in self._executors.items() if k[0] is not fragment}
 
     def set_backend_for_all(self, backend) -> None:
         self._frag_to_backend = {qreg: backend for qreg in self._frag_circs.keys()}
+        self._executors = {}
 
     @staticmethod
     def _replace_vgates_with_endpoints(circuit: QuantumCircuit) -> QuantumCircuit:
@@ -221,10 +224,28 @@ class VirtualCircuit:
         return self._programs[fragment]
 
     def executor(self, fragment: Fragment, device, fold: bool = True) -> FragmentExecutor:
-        key = (fragment, str(device), fold)
+        """The fragment's executor: its density-matrix program (``density.py``) when the fragment is bound to a
+        ``B200Backend(noise_model=...)``, its state-vector program otherwise.  Both fill the same table layout."""
+        model = self.noise_model(fragment)
+        # keyed on the model and its revision too: a backend's model can be swapped or extended between runs
+        key = (fragment, str(device), fold, model, None if model is None else model.revision)
         if key not in self._executors:
-            self._executors[key] = FragmentExecutor(self.program(fragment), device, fold)
+            if model is not None:
+                from .density import DensityExecutor, DensityProgram
+                prog = DensityProgram(self._frag_circs[fragment], fragment, self.num_clbits, model)
+                self._executors[key] = DensityExecutor(prog, device, fold)
+            else:
+                self._executors[key] = FragmentExecutor(self.program(fragment), device, fold)
         return self._executors[key]
+
+    def noise_model(self, fragment: Fragment):
+        """The noise model of the ``B200Backend`` the fragment is bound to (None: noiseless or a foreign backend)."""
+        return getattr(self._frag_to_backend[fragment], "noise_model", None) if isinstance(
+            self._frag_to_backend[fragment], _b200_backend_type()) else None
+
+    def noisy_fragments(self) -> list[Fragment]:
+        """Active fragments bound to a ``B200Backend(noise_model=...)``."""
+        return [f for f in self.active_fragments() if self.noise_model(f) is not None]
 
     def active_fragments(self) -> list[Fragment]:
         """Fragments whose instances measure something (``run.py:49-58`` drops the others)."""
@@ -599,6 +620,11 @@ def _faithful_gate(vg) -> "_lib.QckFaithfulGate":
         g.degenerate = 1 if abs(c) < RZZ_ACCURACY else 2 if abs(s_) < RZZ_ACCURACY else 0
         g.cos_half, g.sin_half, g.cos_half_sq, g.sin_half_sq = c, s_, c ** 2, s_ ** 2
     return g
+
+
+def _b200_backend_type():
+    from .backend import B200Backend
+    return B200Backend
 
 
 def _compress_mask(mask: int, union: int) -> int:

@@ -450,6 +450,53 @@ QCK_API int qck_rows_sample(qck_handle* h, const double* d_in, int64_t n_rows, i
                             double* d_out, int64_t out_row_stride, int fold_bits, int64_t* d_shot_list,
                             uint64_t* d_status, qck_stream stream);
 
+/* ------------------------------------------------------------------ density-matrix simulation under noise
+ * Replaces: backend.run(instantiations, shots) on a noisy Aer backend (run.py:42) by the exact noisy outcome
+ * distribution of every instance (density.py lowers a fragment and a noise model into this plan).
+ *
+ * rho: 2^(2n) complex128, index r | c << n for rho[r][c].  Op record (int32[12]): {nq, mat_off, sel_digit, branch_bit,
+ * p0, p1, p2, p3, s0, s1, s2, s3}: a superoperator (4x4 when nq = 1 on tile positions (p0, p1) = (row bit, column
+ * bit); 16x16 when nq = 2 on (p0, p1, p2, p3) = (r0, r1, c0, c1)), s = the same positions ascending.  Its matrix is
+ * d_mats + mat_off + msize * (digit * (branch_bit >= 0 ? 2 : 1) + bit), digit = the item's label digit sel_digit
+ * (0 when < 0), bit = the item's branch bit branch_bit (0 when < 0), msize = 16 or 256 complex entries.
+ * Sweep: ops [op_begin, op_end) on the tile of entries whose bits outside pos[0..n_tile) are fixed; pos ascending,
+ * pos[k] = k for k < min(5, n_tile).  n_tile = 2n (one sweep, rho never leaves shared memory) when 2n <= 12, else 12.
+ * Item (24 bytes): {uint64 digits (4 bits per digit), int32 label, uint32 branch, uint32 col_base, uint32 qmask};
+ * items are sorted by label and item_begin (HOST, n_labels + 1) indexes them.  An item starts from |0><0|, runs
+ * every sweep and adds Re rho[i][i] to column col_base | sum_{q in qmask} bit_q(i) << qcol[q] of its label's
+ * unfolded row (2^n_cols columns); the items of one label write disjoint columns.  Then every row of
+ * [label_begin, label_end) gets, for each column bit j of d_ro_mask[label], the butterfly
+ * (u0, u1) -> (R00 u0 + R01 u1, R10 u0 + R11 u1) with R = d_ro[j][v] (R[o][i] = p(recorded o | measured i); v = the
+ * label's digit of a configuration column, 0 for a clbit column), and
+ * with fold_bits = f > 0 the top f column bits are folded with sign (-1)^bit into d_out.
+ * d_out row `label` (absolute, stride out_row_stride) receives the result; d_rows (NULL when fold_bits = 0: d_out
+ * is used) holds the unfolded rows of the range, row label - label_begin, stride 2^n_cols.  d_work: as many rho as
+ * fit when 2n > 12 (at least one, else QCK_ERR_NOMEM before anything is launched); unused otherwise. */
+#define QCK_DM_MAX_TILE_BITS 12
+#define QCK_DM_MAX_QUBITS 20
+typedef struct {
+    int32_t n_tile, op_begin, op_end;
+    int32_t pos[QCK_DM_MAX_TILE_BITS];
+} qck_dm_sweep;
+typedef struct {
+    int32_t n_qubits, n_sweeps;
+    const qck_dm_sweep* sweeps;          /* HOST */
+    const int32_t* d_ops;
+    const double* d_mats;                /* complex128 pool */
+    const void* d_items;
+    const int64_t* item_begin;           /* HOST */
+    int64_t n_labels;
+    const uint32_t* d_ro_mask;
+    const double* d_ro;                  /* [n_cols][QCK_MAX_VARIANTS][4] */
+    int32_t n_cols, fold_bits;
+    int32_t qcol[QCK_DM_MAX_QUBITS];
+    int32_t n_digits;                    /* the top n_digits columns are configuration bits */
+    int32_t radix[QCK_MAX_DIGITS];       /* label = mixed radix, last digit fastest */
+} qck_dm_plan;
+QCK_API int qck_sim_density(qck_handle* h, const qck_dm_plan* plan, int64_t label_begin, int64_t label_end,
+                            double* d_out, int64_t out_row_stride, double* d_rows, void* d_work, size_t work_bytes,
+                            qck_stream stream);
+
 /* ------------------------------------------------------------------ reductions
  * qck_stats_dense: sum / min / nnz of a dense vector (entries |v| <= acc count as absent).
  * qck_hellinger: result[0..2] = sum p, sum q, sum sqrt(p q) over max(.,0) entries; the
