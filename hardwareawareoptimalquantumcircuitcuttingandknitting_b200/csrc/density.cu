@@ -270,6 +270,9 @@ QCK_API int qck_sim_density(qck_handle* h, const qck_dm_plan* plan, int64_t labe
     if (out_row_stride < (1ll << (plan->n_cols - plan->fold_bits)) && label_end - label_begin > 1)
         QCK_FAIL(h, QCK_ERR_INVALID_ARG, "output row stride shorter than a row");
     const bool resident = n2 <= QCK_DM_MAX_TILE_BITS;
+    if (resident && plan->n_sweeps != 1)
+        QCK_FAIL(h, QCK_ERR_INVALID_ARG, "a plan of %d qubits (2n <= %d) has one sweep, not %d", n,
+                 QCK_DM_MAX_TILE_BITS, plan->n_sweeps);
     for (int s = 0; s < plan->n_sweeps; ++s) {
         const qck_dm_sweep& sw = plan->sweeps[s];
         const int want = resident ? n2 : QCK_DM_MAX_TILE_BITS;
@@ -288,9 +291,10 @@ QCK_API int qck_sim_density(qck_handle* h, const qck_dm_plan* plan, int64_t labe
     DeviceGuard guard(h->device);
     cudaStream_t st = (cudaStream_t)stream;
     DmRows R;
-    R.rows = d_rows ? d_rows : d_out;
-    R.row_stride = d_rows ? (1ll << plan->n_cols) : out_row_stride;
-    R.row_label0 = d_rows ? label_begin : 0;
+    const bool unfolded = d_rows && plan->fold_bits > 0;    // without a fold the rows are d_out's and d_rows is unused
+    R.rows = unfolded ? d_rows : d_out;
+    R.row_stride = unfolded ? (1ll << plan->n_cols) : out_row_stride;
+    R.row_label0 = unfolded ? label_begin : 0;
     const long long n_rows = label_end - label_begin;
     DmRows Z = R;
     Z.rows = R.rows + (label_begin - R.row_label0) * R.row_stride;
@@ -306,8 +310,10 @@ QCK_API int qck_sim_density(qck_handle* h, const qck_dm_plan* plan, int64_t labe
         const size_t smem = ((size_t)16 << n2) + 256 * 16;
         QCK_CUDA(h, cudaFuncSetAttribute(dm_resident_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         const long long grid = std::min<long long>(ie - ib, (long long)h->sm_count * (smem <= 40 * 1024 ? 4 : 2));
-        dm_resident_kernel<<<(unsigned)grid, DM_THREADS, smem, st>>>(plan->d_ops, plan->sweeps[0].op_end, mats,
-                                                                     items + ib, ie - ib, n, R, Q);
+        const qck_dm_sweep& sw = plan->sweeps[0];
+        dm_resident_kernel<<<(unsigned)grid, DM_THREADS, smem, st>>>(plan->d_ops + DM_OP_INTS * sw.op_begin,
+                                                                     sw.op_end - sw.op_begin, mats, items + ib,
+                                                                     ie - ib, n, R, Q);
         QCK_CHECK_LAUNCH(h);
     } else if (ie > ib) {
         const size_t smem = ((size_t)16 << QCK_DM_MAX_TILE_BITS) + 256 * 16;

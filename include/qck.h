@@ -469,7 +469,7 @@ QCK_API int qck_rows_sample(qck_handle* h, const double* d_in, int64_t n_rows, i
  * (u0, u1) -> (R00 u0 + R01 u1, R10 u0 + R11 u1) with R = d_ro[j][v] (R[o][i] = p(recorded o | measured i); v = the
  * label's digit of a configuration column, 0 for a clbit column), and
  * with fold_bits = f > 0 the top f column bits are folded with sign (-1)^bit into d_out.
- * d_out row `label` (absolute, stride out_row_stride) receives the result; d_rows (NULL when fold_bits = 0: d_out
+ * d_out row `label` (absolute, stride out_row_stride) receives the result; d_rows (unused when fold_bits = 0: d_out
  * is used) holds the unfolded rows of the range, row label - label_begin, stride 2^n_cols.  d_work: as many rho as
  * fit when 2n > 12 (at least one, else QCK_ERR_NOMEM before anything is launched); unused otherwise. */
 #define QCK_DM_MAX_TILE_BITS 12
