@@ -435,10 +435,8 @@ extern "C" int qck_knit_faithful_part(qck_handle* h, int n_frag, const double* c
     const unsigned long long total = n_gates ? n * (unsigned long long)(2 * P.radix[0]) : 0;
     size_t tree_bytes = (total * sizeof(double) + 255) & ~(size_t)255, flag_bytes = 0, list_bytes = 0;
     // second split level (sparse path): scratch for the (gate 0, gate 1) subtrees, bounded at 1 GiB
-    const char* split_env = getenv("QCK_FAITHFUL_SPLIT2");
     const unsigned long long total2 = n_gates >= 2 ? total * (unsigned long long)(2 * P.radix[1]) : 0;
-    const bool split2 = sparse && n_gates >= 2 && total2 * sizeof(double) <= ((size_t)1 << 30) &&
-                        !(split_env && atoi(split_env) == 0);
+    const bool split2 = sparse && n_gates >= 2 && total2 * sizeof(double) <= ((size_t)1 << 30);
     const size_t tree1_bytes = tree_bytes;
     if (split2) tree_bytes += (total2 * sizeof(double) + 255) & ~(size_t)255;
     long long list_stride = 0;

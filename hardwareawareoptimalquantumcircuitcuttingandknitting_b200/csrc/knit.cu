@@ -611,64 +611,11 @@ __global__ void __launch_bounds__(256) contract_generic_kernel(const __grid_cons
 // two fragments: C[i][j] = sum_l w[l] A[rowA[l]][i] B[rowB[l]][j]  (64x64 tile, split over l)
 #define GT 64
 #define GK 16
-__global__ void __launch_bounds__(256) contract_gemm_kernel(const __grid_constant__ ContractParams P, int n_split,
-                                                            double* __restrict__ partial, int M, int N, int Mr,
-                                                            int Nr) {
-    __shared__ double As[GK][GT + 4];
-    __shared__ double Bs[GK][GT + 4];
-    const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
-    const int i0 = blockIdx.x * GT, j0 = blockIdx.y * GT;
-    const long long per = (P.count + n_split - 1) / n_split;
-    const long long lb = per * blockIdx.z, le = (lb + per < P.count) ? lb + per : P.count;
-    const int* rowA = P.rows;
-    const int* rowB = P.rows + P.count;
-    double acc[4][4];
-#pragma unroll
-    for (int a = 0; a < 4; ++a)
-#pragma unroll
-        for (int b = 0; b < 4; ++b) acc[a][b] = 0.0;
-    for (long long l0 = lb; l0 < le; l0 += GK) {
-#pragma unroll
-        for (int k = 0; k < (GK * GT) / 256; ++k) {
-            int e = tid + 256 * k, rr = e / GT, cc = e % GT;
-            long long l = l0 + rr;
-            double a = 0.0, b = 0.0;
-            if (l < le) {  // Mr / Nr: real row lengths (a fragment with fewer than 6 output bits fills part of a tile)
-                if (i0 + cc < Mr)
-                    a = __ldg(P.w + l) * __ldg(P.table[0] + (long long)__ldg(rowA + l) * P.row_stride[0] + i0 + cc);
-                if (j0 + cc < Nr) b = __ldg(P.table[1] + (long long)__ldg(rowB + l) * P.row_stride[1] + j0 + cc);
-            }
-            As[rr][cc] = a;
-            Bs[rr][cc] = b;
-        }
-        __syncthreads();
-#pragma unroll
-        for (int kk = 0; kk < GK; ++kk) {
-            double a[4], b[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                a[u] = As[kk][ty * 4 + u];
-                b[u] = Bs[kk][tx * 4 + u];
-            }
-#pragma unroll
-            for (int u = 0; u < 4; ++u)
-#pragma unroll
-                for (int v = 0; v < 4; ++v) acc[u][v] = fma(a[u], b[v], acc[u][v]);
-        }
-        __syncthreads();
-    }
-    double* dst = partial + (long long)blockIdx.z * M * N;
-#pragma unroll
-    for (int u = 0; u < 4; ++u)
-#pragma unroll
-        for (int v = 0; v < 4; ++v) dst[(long long)(i0 + ty * 4 + u) * N + (j0 + tx * 4 + v)] = acc[u][v];
-}
-
-// FP64 tensor-core form of the same tile (sm_100a: mma.sync.aligned.m8n8k4.f64 = DMMA; tcgen05 has
-// no FP64 kind).  64x64 output tile per CTA, 8 warps, each warp owns a 32x16 sub-tile = 4x2 DMMA
-// tiles (16 accumulator registers).  Per k-step of 4 labels a warp issues 8 DMMAs (2048 FMA) against
-// 6 LDS.64 per thread: 0.75 B of shared-memory traffic per FMA instead of 4 B on the FMA-pipe kernel,
-// which was shared-memory bound.  As/Bs rows are padded to 72 doubles so that a fragment load (lanes
+// on FP64 tensor cores (sm_100a: mma.sync.aligned.m8n8k4.f64 = DMMA; tcgen05 has no FP64 kind).
+// 64x64 output tile per CTA, 8 warps, each warp owns a 32x16 sub-tile = 4x2 DMMA tiles (16 accumulator
+// registers).  Per k-step of 4 labels a warp issues 8 DMMAs (2048 FMA) against 6 LDS.64 per thread:
+// 0.75 B of shared-memory traffic per FMA instead of 4 B on an FMA-pipe tile, which was measured
+// shared-memory bound and removed.  As/Bs rows are padded to 72 doubles so that a fragment load (lanes
 // vary the row by lane>>2 and k by lane&3) needs exactly two 128-byte wavefronts.
 #define GP 72
 __device__ __forceinline__ void dmma_m8n8k4(double& c0, double& c1, double a, double b) {
@@ -745,8 +692,8 @@ __global__ void __launch_bounds__(256) contract_dmma_kernel(const __grid_constan
 // Tile size (round 2, second half): at 64x64 every 16-label chunk brings 16 KiB from L2 for 131 kflop - 8 flop per
 // gathered byte, which makes the kernel an L2-gather kernel (ncu: DMMA 41 % of its peak on hwe-16 d5's 256x256
 // output, 304 CTAs each re-reading a quarter of both tables).  TT = 128 halves the bytes per flop and quarters the
-// barriers per flop: 16 warps of 32x32 (4x4 DMMA tiles, 8 LDS.64 for 16 DMMAs per k-step; or 8 warps of 64x32),
-// one CTA per SM.  Used when both padded dimensions are multiples of 128 and there are at least 4096 labels.
+// barriers per flop: 16 warps of 32x32 (4x4 DMMA tiles, 8 LDS.64 for 16 DMMAs per k-step; the DMMA pipe 61 % busy
+// on hwe-16 d5, against 59 % with 8 warps of 64x32, which were removed), one CTA per SM.  Used when both padded dimensions are multiples of 128 and there are at least 4096 labels.
 #define GS 3
 template <int TT>
 struct ContractStage {
@@ -1127,32 +1074,21 @@ extern "C" int qck_knit_contract(qck_handle* h, int n_frag, const double* const*
     if (gemm && full_cover) {
         const int M = 1 << mAp, N = 1 << mBp, Mr = 1 << mA, Nr = 1 << mB;
         dim3 grid(M / GT, N / GT, n_split);
-        // FP64 tensor cores (DMMA) by default; QCK_CONTRACT_FMA=1 selects the FMA-pipe tile kernel
-        const char* fma_env = getenv("QCK_CONTRACT_FMA");
         // pipelined gather (cp.async, 16-byte requests): rows must start on 16-byte boundaries and be even
         const char* pipe_env = getenv("QCK_CONTRACT_PIPE");
         const bool aligned = ((reinterpret_cast<uintptr_t>(tabs[0]) | reinterpret_cast<uintptr_t>(tabs[1])) & 15) == 0 &&
                              ((rstr[0] | rstr[1]) & 1) == 0 && Mr >= 2 && Nr >= 2;
-        if (fma_env && atoi(fma_env) == 1)
-            contract_gemm_kernel<<<grid, 256, 0, st>>>(cp, n_split, d_partial, M, N, Mr, Nr);
-        else if (aligned && !(pipe_env && atoi(pipe_env) == 0)) {
+        if (aligned && !(pipe_env && atoi(pipe_env) == 0)) {
             static bool attr_set = false;  // process-wide function attributes, same values from every thread
             if (!attr_set) {
                 QCK_CUDA(h, cudaFuncSetAttribute(contract_dmma_pipe_kernel<64, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                                  (int)(GS * sizeof(ContractStage<64>))));
-                QCK_CUDA(h, cudaFuncSetAttribute(contract_dmma_pipe_kernel<128, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                 (int)(GS * sizeof(ContractStage<128>))));
                 QCK_CUDA(h, cudaFuncSetAttribute(contract_dmma_pipe_kernel<128, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                                  (int)(GS * sizeof(ContractStage<128>))));
                 attr_set = true;
             }
-            const char* warps_env = getenv("QCK_CONTRACT_WARPS");
-            // 16 warps of 32x32 by default (DMMA pipe 61 % busy on hwe-16 d5, 59 % with 8 warps of 64x32: QCK_CONTRACT_WARPS=8)
-            if (big_tile && !(warps_env && atoi(warps_env) == 8))
+            if (big_tile)
                 contract_dmma_pipe_kernel<128, 16><<<dim3(M / 128, N / 128, n_split), 512, GS * sizeof(ContractStage<128>), st>>>(
-                    cp, n_split, d_partial, M, N, Mr, Nr);
-            else if (big_tile)
-                contract_dmma_pipe_kernel<128, 8><<<dim3(M / 128, N / 128, n_split), 256, GS * sizeof(ContractStage<128>), st>>>(
                     cp, n_split, d_partial, M, N, Mr, Nr);
             else
                 contract_dmma_pipe_kernel<64, 8><<<grid, 256, GS * sizeof(ContractStage<64>), st>>>(cp, n_split, d_partial, M, N,

@@ -433,140 +433,6 @@ __global__ void __launch_bounds__(NPD_THREADS) npd_apply_kernel(double* __restri
     }
 }
 
-// ---- small vectors: the whole search as ONE cooperative launch.  At 2^16 entries (every 16-qubit configuration)
-// each of the eight launches above lasts 5-14 us and does microseconds of work; here the passes are separated by
-// grid-wide barriers instead of launches, CTA 0 runs the tails, and the level loop stops as soon as the partition
-// is located instead of enqueueing every level unconditionally.  Same arithmetic in the same order: same bits.
-__global__ void __launch_bounds__(NPD_THREADS) npd_fused_kernel(double* __restrict__ p, unsigned long long n, double acc,
-                                                                void* ws_raw) {
-    namespace cg = cooperative_groups;
-    cg::grid_group grid = cg::this_grid();
-    NpdWs w = npd_ws(ws_raw);
-    __shared__ double red[8];
-    unsigned int* h_cnt = reinterpret_cast<unsigned int*>(npd_smem);
-    unsigned long long* h_q = reinterpret_cast<unsigned long long*>(npd_smem + 4 * NPD_BINS);
-    const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
-    const unsigned long long first = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
-    // pass 1: statistics
-    {
-        double s = 0.0, m = INFINITY, ns = 0.0, z = 0.0, nz = 0.0;
-        for (unsigned long long i = first; i < n; i += stride) {
-            const double v = p[i];
-            if (fabs(v) > acc) {
-                s += v;
-                m = fmin(m, v);
-                z += 1.0;
-                if (v < 0.0) {
-                    ns += v;
-                    nz += 1.0;
-                }
-            }
-        }
-        s = block_sum(s, red);
-        m = block_min(m, red);
-        ns = block_sum(ns, red);
-        z = block_sum(z, red);
-        nz = block_sum(nz, red);
-        if (threadIdx.x == 0) {
-            double* o = w.partials + 8 * blockIdx.x;
-            o[0] = s; o[1] = m; o[2] = ns; o[3] = z; o[4] = nz;
-        }
-    }
-    grid.sync();
-    if (blockIdx.x == 0) {
-        double s = 0.0, m = INFINITY, ns = 0.0, z = 0.0, nz = 0.0;
-        for (int i = threadIdx.x; i < (int)gridDim.x; i += blockDim.x) {
-            const double* o = w.partials + 8 * i;
-            s += __ldcg(o + 0); m = fmin(m, __ldcg(o + 1)); ns += __ldcg(o + 2); z += __ldcg(o + 3); nz += __ldcg(o + 4);
-        }
-        s = block_sum(s, red);
-        m = block_min(m, red);
-        ns = block_sum(ns, red);
-        z = block_sum(z, red);
-        nz = block_sum(nz, red);
-        if (threadIdx.x == 0) {
-            w.st->sum = s; w.st->vmin = m; w.st->neg_sum = ns; w.st->alive = z; w.st->neg_cnt = nz;
-        }
-        __syncthreads();
-        npd_plan_tail(w);
-    }
-    grid.sync();
-    // levels (+ the final pass that takes (sum, count) of the dropped entries)
-    for (int level = 0; level <= NPD_LEVELS + 1; ++level) {
-        const int status = (int)__ldcg(&w.st->status);  // written by CTA 0 before the barrier: read past L1
-        if (status != NPD_SEARCH && status != NPD_LOCATED) break;
-        const bool bins = status == NPD_SEARCH;
-        if (bins)
-            for (int i = threadIdx.x; i < NPD_BINS; i += blockDim.x) {
-                h_cnt[i] = 0u;
-                h_q[i] = 0ull;
-            }
-        const long long lo = __ldcg(&w.st->lo), hi = __ldcg(&w.st->hi);
-        const int shift = (int)__ldcg(&w.st->shift);
-        const double lo_val = npd_val(lo + 1);
-        const int qexp = (int)__ldcg(&w.st->qexp);
-        __syncthreads();
-        double us = 0.0, uc = 0.0;
-        for (unsigned long long i = first; i < n; i += stride) {
-            const double v = p[i];
-            if (!(fabs(v) > acc)) continue;
-            const long long k = npd_key(v);
-            if (k <= lo) {
-                us += v;
-                uc += 1.0;
-            } else if (bins && k <= hi) {
-                const unsigned int b = (unsigned int)(((unsigned long long)k - (unsigned long long)lo - 1ull) >> shift);
-                atomicAdd(&h_cnt[b], 1u);
-                atomicAdd(&h_q[b], (unsigned long long)__double2ll_rn(scalbn(v - lo_val, qexp)));
-            }
-        }
-        us = block_sum(us, red);
-        uc = block_sum(uc, red);
-        if (threadIdx.x == 0) {
-            w.partials[8 * blockIdx.x + 0] = us;
-            w.partials[8 * blockIdx.x + 1] = uc;
-        }
-        if (bins) {
-            __syncthreads();
-            for (int i = threadIdx.x; i < NPD_BINS; i += blockDim.x) {
-                const unsigned int c = h_cnt[i];
-                if (c) {
-                    atomicAdd(&w.bin_cnt[i], (unsigned long long)c);
-                    atomicAdd(reinterpret_cast<unsigned long long*>(&w.bin_q[i]), h_q[i]);
-                }
-            }
-        }
-        grid.sync();
-        if (blockIdx.x == 0) {
-            us = 0.0;
-            uc = 0.0;
-            for (int i = threadIdx.x; i < (int)gridDim.x; i += blockDim.x) {
-                us += __ldcg(w.partials + 8 * i + 0);
-                uc += __ldcg(w.partials + 8 * i + 1);
-            }
-            us = block_sum(us, red);
-            uc = block_sum(uc, red);
-            if (threadIdx.x == 0) {
-                w.st->under_sum = us;
-                w.st->under_cnt = uc;
-            }
-            __syncthreads();
-            npd_select_tail(w);
-        }
-        grid.sync();
-    }
-    // apply
-    const int status = (int)__ldcg(&w.st->status);
-    if (status == NPD_IDENTITY && !(acc > 0.0)) return;
-    if (status != NPD_IDENTITY && status != NPD_SOLVED) return;
-    const long long lo = status == NPD_SOLVED ? __ldcg(&w.st->lo) : (long long)0x8000000000000000ull;
-    const double shift_val = status == NPD_SOLVED ? __ldcg(&w.st->shift_val) : 0.0;
-    for (unsigned long long i = first; i < n; i += stride) {
-        const double v = p[i];
-        p[i] = (fabs(v) > acc && npd_key(v) > lo) ? v + shift_val : 0.0;
-    }
-}
-
 // ---- vectors of at most 2^16 entries (every 16-qubit configuration): the whole search as ONE launch of ONE
 // thread-block cluster.  Eight CTAs hold the vector in registers (16 entries per thread); the passes are separated
 // by cluster barriers instead of launches; the bins (2048 per level: 11 key bits) live in shared memory.  After a
@@ -619,17 +485,13 @@ __device__ __forceinline__ void npc_block_reduce(double (&x)[N], NpcShared& S, d
 }
 
 __global__ void __cluster_dims__(NPC_CTAS, 1, 1) __launch_bounds__(NPC_THREADS)
-    npd_cluster_kernel(double* __restrict__ p, unsigned long long n, double acc, void* ws_raw, int mode) {
+    npd_cluster_kernel(double* __restrict__ p, unsigned long long n, double acc, void* ws_raw) {
     namespace cg = cooperative_groups;
     cg::cluster_group cluster = cg::this_cluster();
     NpcShared& S = *reinterpret_cast<NpcShared*>(npd_smem);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const unsigned int rank = cluster.block_rank();
     NpdState* s = &S.st;
-    long long tmark[12];
-    int nmark = 0;
-#define NPC_MARK() do { if (nmark < 12) tmark[nmark++] = clock64(); } while (0)
-    NPC_MARK();
 
     // the vector, 16 entries per thread (entry i of the vector: CTA i / 8192, then coalesced)
     double v[NPC_VPT];
@@ -680,14 +542,13 @@ __global__ void __cluster_dims__(NPC_CTAS, 1, 1) __launch_bounds__(NPC_THREADS)
         } else {
             s->status = NPD_SEARCH;
             // G(0) = neg_sum < 0: t0 > 0, every entry <= 0 is dropped - the search starts above zero
-            s->lo = (mode & 32) ? npd_key(m) - 1 : 0ll;
+            s->lo = 0ll;
             s->hi = npd_key(-ns * (1.0 + 1e-9));
             s->sel_cnt = (long long)z;
             npd_set_level(s, NPC_BIN_BITS);
         }
     }
     cluster.sync();  // (also: S.part has been read by every CTA before the first pass overwrites it)
-    NPC_MARK();
 
     for (int level = 0; level <= NPC_LEVELS + 1; ++level) {
         const int status = (int)s->status;
@@ -731,7 +592,6 @@ __global__ void __cluster_dims__(NPC_CTAS, 1, 1) __launch_bounds__(NPC_THREADS)
             }
         }
         npc_block_reduce<2>(x, S, S.part, false);
-        NPC_MARK();
         cluster.sync();  // bins and partial sums of every CTA are complete
         if (tid < NPC_CTAS * 2) S.gathered[tid] = cluster.map_shared_rank(S.part, tid / 2)[tid % 2];
         unsigned int c_bin = 0u;
@@ -788,10 +648,8 @@ __global__ void __cluster_dims__(NPC_CTAS, 1, 1) __launch_bounds__(NPC_THREADS)
         }
         if (!bins) {
             __syncthreads();
-            NPC_MARK();
             continue;  // every CTA has computed the same state
         }
-        NPC_MARK();
         cluster.sync();  // slice totals
         if (tid < NPC_CTAS * 2) S.gathered_slices[tid] = cluster.map_shared_rank(S.slice_tot, tid / 2)[tid % 2];
         __syncthreads();
@@ -858,7 +716,6 @@ __global__ void __cluster_dims__(NPC_CTAS, 1, 1) __launch_bounds__(NPC_THREADS)
                     reinterpret_cast<const long long*>(s)[tid % SLOTS];
         }
         cluster.sync();  // new state everywhere
-        NPC_MARK();
     }
     // apply
     const int status = (int)s->status;
@@ -873,11 +730,7 @@ __global__ void __cluster_dims__(NPC_CTAS, 1, 1) __launch_bounds__(NPC_THREADS)
     }
     if (rank == 0 && tid < (int)(sizeof(NpdState) / 8) && tid != 17)  // (slot 17 = the ticket of the staged kernels)
         reinterpret_cast<long long*>(ws_raw)[tid] = reinterpret_cast<const long long*>(s)[tid];
-    NPC_MARK();
-    if (rank == 0 && tid == 0 && (mode & 64))
-        for (int i = 0; i < 12; ++i) reinterpret_cast<long long*>(ws_raw)[19 + i] = i < nmark ? tmark[i] - tmark[0] : -1;
     cluster.sync();  // no CTA leaves while its shared memory may still be read
-#undef NPC_MARK
 }
 
 // ------------------------------------------------------------------ host side
@@ -892,7 +745,6 @@ static int npd_grid(qck_handle* h, unsigned long long n) {
 
 int qck_npd_init(qck_handle* h) {
     QCK_CUDA(h, cudaFuncSetAttribute(npd_hist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 12 * NPD_BINS));
-    QCK_CUDA(h, cudaFuncSetAttribute(npd_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 12 * NPD_BINS));
     QCK_CUDA(h, cudaFuncSetAttribute(npd_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(NpcShared)));
     QCK_CUDA(h, cudaMalloc(&h->npd_ws, NPD_WS_BYTES));
     QCK_CUDA(h, cudaMemset(h->npd_ws, 0, NPD_WS_BYTES));
@@ -925,30 +777,14 @@ extern "C" int qck_npd_stage(qck_handle* h, int stage, double* d_p, uint64_t n, 
 extern "C" int qck_npd_async(qck_handle* h, double* d_p, uint64_t n, double acc, void* d_ws, qck_stream stream) {
     if (!h) return QCK_ERR_INVALID_ARG;
     if (!d_p && n > 0) QCK_FAIL(h, QCK_ERR_INVALID_ARG, "NULL argument");
-    // QCK_NPD_FUSED=1: one cooperative launch while all CTAs of the grid are co-resident with room to spare.
-    // Opt-in: measured on hwe-16 d5 / bv-16 (2^16 entries, inside the step's CUDA graph) it saves 2-4 us of the
-    // 75 / 53 us the eight launches take - the passes themselves, not the launches, are the cost - which does not
-    // pay for depending on cooperative launches inside captured graphs.
     // n <= 2^16: one launch of one 8-CTA cluster, the vector in registers, bins in (distributed) shared memory
     // (QCK_NPD_CLUSTER=0: the staged launches below)
     const char* cluster_env = getenv("QCK_NPD_CLUSTER");
     if (n <= NPC_CAPACITY && !(cluster_env && atoi(cluster_env) == 0)) {
         DeviceGuard guard(h->device);
         void* ws = d_ws ? d_ws : h->npd_ws;
-        const char* mode_env = getenv("QCK_NPC_MODE");
-        npd_cluster_kernel<<<NPC_CTAS, NPC_THREADS, sizeof(NpcShared), (cudaStream_t)stream>>>(d_p, n, acc, ws, mode_env ? atoi(mode_env) : 0);  // (debug bits: 32 = the staged kernels' first range, 64 = cycle marks into slots 19-30)
+        npd_cluster_kernel<<<NPC_CTAS, NPC_THREADS, sizeof(NpcShared), (cudaStream_t)stream>>>(d_p, n, acc, ws);
         QCK_CHECK_LAUNCH(h);
-        return QCK_OK;
-    }
-    const char* fused_env = getenv("QCK_NPD_FUSED");
-    if (n > 0 && npd_grid(h, n) <= h->sm_count && fused_env && atoi(fused_env) == 1) {
-        DeviceGuard guard(h->device);
-        void* ws = d_ws ? d_ws : h->npd_ws;
-        unsigned long long nn = n;
-        void* args[] = {&d_p, &nn, &acc, &ws};
-        QCK_CUDA(h, cudaLaunchCooperativeKernel((const void*)npd_fused_kernel, dim3(npd_grid(h, n)), dim3(NPD_THREADS), args,
-                                                12 * NPD_BINS, (cudaStream_t)stream));
-        h->launches++;
         return QCK_OK;
     }
     int rc = qck_npd_stage(h, QCK_NPD_STATS, d_p, n, acc, d_ws, 1, stream);

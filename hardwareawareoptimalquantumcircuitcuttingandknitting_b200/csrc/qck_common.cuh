@@ -17,7 +17,7 @@ struct qck_handle {
     int64_t launches;
     char err[512];
     // small device scratch for reductions (per-CTA partials); the last 8 doubles are reserved for the
-    // streaming simulator (instance label, tile counter) and never handed out by qck_ensure_partials
+    // streaming simulator (instance label) and never handed out by qck_ensure_partials
     double* d_partials;
     size_t partials_count;
     // pinned host scratch for scalar read-backs

@@ -1263,10 +1263,9 @@ static int run_sweeps(qck_handle* h, const qck_sim_plan* plan, const PlanDev& pd
     }
     if (use_tma) {
         unsigned long long live = 0;
-        // The dead region is zero-filled by a streaming kernel up front (QCK_TMA_PREZERO=0: by the last sweep
-        // itself, tile by tile, as in round 1); the last sweep then visits the live tiles only.
+        // The dead region is zero-filled by a streaming kernel up front; the last sweep then visits the live tiles
+        // only.  (The sharded sweeps instead have their last sweep write the dead tiles: skip_dead = false.)
         bool prezero = true;
-        if (const char* env = getenv("QCK_TMA_PREZERO")) prezero = atoi(env) != 0;
         {
             unsigned long long live_after = 0;
             for (int i = 0; i < plan->n_sweeps; ++i)
@@ -1280,11 +1279,9 @@ static int run_sweeps(qck_handle* h, const qck_sim_plan* plan, const PlanDev& pd
                 if (rc) return rc;
             }
         }
-        // Tile scheduling: static round robin by default.  Pulling tiles from a counter (QCK_TMA_DYNAMIC=1)
-        // measured 1-2 % faster on compute-heavy sweeps but 13 % slower on the write-only expansion sweep
-        // of syc-32 d1 (15.1 vs 13.4 ms): neighbouring CTAs on neighbouring tiles suit the TMA stores.
-        int tma_dynamic = 0;
-        if (const char* env = getenv("QCK_TMA_DYNAMIC")) tma_dynamic = atoi(env);
+        // Tile scheduling: static round robin.  Pulling tiles from a counter measured 1-2 % faster on
+        // compute-heavy sweeps but 13 % slower on the write-only expansion sweep of syc-32 d1 (15.1 vs
+        // 13.4 ms): neighbouring CTAs on neighbouring tiles suit the TMA stores.
         for (int i = 0; i < plan->n_sweeps; ++i) {
             tma_describe(plan, i, live, i == plan->n_sweeps - 1, batch, h->max_smem_optin, *L, nullptr, prezero);
             for (int j = 0; j < plan->sweeps[i].n_tile; ++j) live |= 1ull << plan->sweeps[i].pos[j];
@@ -1303,17 +1300,12 @@ static int run_sweeps(qck_handle* h, const qck_sim_plan* plan, const PlanDev& pd
             PlanDev pdl = pd;
             pdl.n_stage = L->n_stage;
             unsigned long long grid = L->n_work < (unsigned long long)h->sm_count ? L->n_work : (unsigned long long)h->sm_count;
-            unsigned long long* counter = nullptr;
-            if (tma_dynamic && L->n_work > grid && !h->region) {  // reserved tail of the reduction scratch (qck_common.cuh)
-                counter = reinterpret_cast<unsigned long long*>(h->d_partials + h->partials_count - 4);
-                QCK_CUDA(h, cudaMemsetAsync(counter, 0, sizeof(unsigned long long), st));
-            }
             if (L->sd.n_store >= 16 || L->sd.n_load >= 16)  // measured: 8 boxes of 8 KiB are still faster from one lane
                 sim_sweep_tma_wide_kernel<<<(unsigned)grid, TMA_CONSUMERS + 32, L->smem, st>>>(
-                    L->maps, L->sd, pdl, d_labels, inst_base, L->n_work, counter);
+                    L->maps, L->sd, pdl, d_labels, inst_base, L->n_work);
             else
                 sim_sweep_tma_kernel<<<(unsigned)grid, TMA_CONSUMERS + 32, L->smem, st>>>(
-                    L->maps, L->sd, pdl, d_labels, inst_base, L->n_work, counter);
+                    L->maps, L->sd, pdl, d_labels, inst_base, L->n_work);
             QCK_CHECK_LAUNCH(h);
         }
         return QCK_OK;
@@ -1332,13 +1324,9 @@ static int run_sweeps(qck_handle* h, const qck_sim_plan* plan, const PlanDev& pd
         unsigned long long tiles = 1ull << (plan->n_state_qubits - sd.n_tile);
         if (tiles > 0x7fffffffull) QCK_FAIL(h, QCK_ERR_UNSUPPORTED, "too many tiles");
         dim3 grid((unsigned)tiles, (unsigned)batch);
+        // many tiles: 128 threads, 3 CTAs per SM de-phase load / compute / store (256 threads: 2 phase-locked CTAs);
         // few tiles (L2-resident states): latency bound, use all 256 threads per tile
-        int sweep_threads = tiles * (unsigned long long)batch >= 4ull * h->sm_count ? 128 : 256;  // 3 CTAs per SM de-phase load / compute / store (256 threads: 2 phase-locked CTAs);
-        //                           QCK_SWEEP_THREADS overrides (tuning knob; multiple of 64)
-        if (const char* env = getenv("QCK_SWEEP_THREADS")) {
-            int v = atoi(env);
-            if (v >= 64 && v <= 256 && v % 64 == 0) sweep_threads = v;
-        }
+        const int sweep_threads = tiles * (unsigned long long)batch >= 4ull * h->sm_count ? 128 : 256;
         sim_sweep_kernel<<<grid, sweep_threads, smem, st>>>(pdl, sd, d_labels, inst_base, work, state_stride);
         QCK_CHECK_LAUNCH(h);
     }
@@ -1471,16 +1459,7 @@ static int qck_warp_init(qck_handle* h) {
     return QCK_OK;
 }
 
-static int warp_dfs_levels() {  // QCK_WARP_DFS_LEVELS: outcome levels one warp walks itself (tuning knob)
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("QCK_WARP_DFS_LEVELS");
-        v = e ? atoi(e) : 2;
-        if (v < 0) v = 0;
-        if (v > QCK_WARP_MAX_DEPTH) v = QCK_WARP_MAX_DEPTH;
-    }
-    return v;
-}
+#define WARP_DFS_LEVELS 2  // outcome levels one warp walks itself; the levels above are split over warps
 
 // A group of register-resident plans (same fragment qubit count) = one launch.  warp_group_layout fills the
 // kernel parameters and says how much scratch the launch needs ([global stash | partial rows | counters]);
@@ -1538,7 +1517,7 @@ static int warp_group_layout(qck_handle* h, const qck_sim_plan* plans, const int
         v.sum_mask = p.sum_mask;
         v.sign_mask = p.sign_mask;
         v.labels = d_labels[idx[i]];
-        v.split_bits = (v.mode == QCK_WARP_MODE_ACC && n_anc > warp_dfs_levels()) ? n_anc - warp_dfs_levels() : 0;
+        v.split_bits = (v.mode == QCK_WARP_MODE_ACC && n_anc > WARP_DFS_LEVELS) ? n_anc - WARP_DFS_LEVELS : 0;
         const int walk = n_anc - v.split_bits;
         if (walk > max_walk) max_walk = walk;
         v.item_begin = (int)items;
@@ -1672,6 +1651,8 @@ extern "C" size_t qck_sim_tree_work_bytes(const qck_sim_tree_plan* plan) {
     return 2 * sb + pb;
 }
 
+#define TREE_FUSE_ITEMS 300  // items of the last level fused into the first launch of qck_sim_tree
+
 extern "C" int qck_sim_tree(qck_handle* h, const qck_sim_tree_plan* plan, int64_t label_begin, int64_t label_end,
                             double* d_out, int64_t out_row_stride, void* d_work, size_t work_bytes,
                             qck_stream stream) {
@@ -1729,22 +1710,16 @@ extern "C" int qck_sim_tree(qck_handle* h, const qck_sim_tree_plan* plan, int64_
     double2* sbuf[2] = {reinterpret_cast<double2*>(d_work), reinterpret_cast<double2*>((char*)d_work + sb)};
     double* part = reinterpret_cast<double*>((char*)d_work + 2 * sb);
     const long long cap = (long long)h->sm_count * h->tree_occ[log_r];
-    int dbg_skip = 0;
-    if (const char* e = getenv("QCK_TREE_DEBUG_SKIP")) dbg_skip = atoi(e);  // timing experiments only
     // the first levels in ONE launch (every warp replays its item's path from the root) while the last fused
-    // level has at most 300 items; QCK_TREE_FUSE_ITEMS overrides the limit (0: one launch per level).  Measured:
+    // level has at most TREE_FUSE_ITEMS items.  Measured:
     // hwe-16 d5 0.1735 -> 0.1689 ms, syc-16 d5 0.119 -> 0.113 ms per step with levels 0-2 (216 items) fused; fusing
     // on to 1 296 items (one wave of warps) gives the gain back - a level is bound by its chain of gates, not by
     // its launch, and the replay makes the chain longer.
-    long long fuse_cap = 300;
+    long long fuse_cap = TREE_FUSE_ITEMS;
     if (fuse_cap > cap * QCK_WARP_PER_CTA) fuse_cap = cap * QCK_WARP_PER_CTA;
-    if (const char* e = getenv("QCK_TREE_FUSE_ITEMS")) fuse_cap = atoll(e);
     int fused_to = 0;
     while (fused_to + 1 < plan->n_levels && n[fused_to + 2] <= fuse_cap) ++fused_to;
-    if (dbg_skip) fused_to = 0;
     for (int l = fused_to; l < plan->n_levels; ++l) {
-        if ((dbg_skip & 2) && l == plan->n_levels - 1) continue;
-        if ((dbg_skip & 4) && l < plan->n_levels - 1) continue;
         const long long items = n[l + 1];
         long long ctas = (items + QCK_WARP_PER_CTA - 1) / QCK_WARP_PER_CTA;
         if (ctas > cap) ctas = cap;
@@ -1772,13 +1747,11 @@ extern "C" int qck_sim_tree(qck_handle* h, const qck_sim_tree_plan* plan, int64_
     }
     if (n_fork_max > 8) QCK_FAIL(h, QCK_ERR_UNSUPPORTED, "more than 8 measuring slots whose qubit lives on");
     if (n_eq_max > 256) QCK_FAIL(h, QCK_ERR_UNSUPPORTED, "more than 256 labels share one representative");
-    if (!(dbg_skip & 1)) {
-        unsigned long long cg = ((unsigned long long)n_rep_labels + QCK_TREE_COMBINE_WARPS - 1) / QCK_TREE_COMBINE_WARPS;
-        if (cg > (unsigned long long)h->sm_count * 8) cg = (unsigned long long)h->sm_count * 8;
-        sim_tree_combine_kernel<<<(unsigned)cg, 32 * QCK_TREE_COMBINE_WARPS, 0, st>>>(
-            *T, n_rep_labels, label_begin, label_end, part, d_out, (long long)out_row_stride);
-        QCK_CHECK_LAUNCH(h);
-    }
+    unsigned long long cg = ((unsigned long long)n_rep_labels + QCK_TREE_COMBINE_WARPS - 1) / QCK_TREE_COMBINE_WARPS;
+    if (cg > (unsigned long long)h->sm_count * 8) cg = (unsigned long long)h->sm_count * 8;
+    sim_tree_combine_kernel<<<(unsigned)cg, 32 * QCK_TREE_COMBINE_WARPS, 0, st>>>(
+        *T, n_rep_labels, label_begin, label_end, part, d_out, (long long)out_row_stride);
+    QCK_CHECK_LAUNCH(h);
     return QCK_OK;
 }
 
@@ -2142,10 +2115,10 @@ extern "C" int qck_sim_sweeps_sharded(qck_handle* h, const qck_sim_plan* plan, i
                     L->n_work < (unsigned long long)h->sm_count ? L->n_work : (unsigned long long)h->sm_count;
                 if (L->sd.n_store >= 16 || L->sd.n_load >= 16)  // measured: 8 boxes of 8 KiB are still faster from one lane
                     sim_sweep_tma_sharded_wide_kernel<<<(unsigned)grid, TMA_CONSUMERS + 32, L->smem, st>>>(
-                        L->maps, L->sd, pdl, d_label, 0, L->n_work, nullptr);
+                        L->maps, L->sd, pdl, d_label, 0, L->n_work);
                 else
                     sim_sweep_tma_sharded_kernel<<<(unsigned)grid, TMA_CONSUMERS + 32, L->smem, st>>>(
-                        L->maps, L->sd, pdl, d_label, 0, L->n_work, nullptr);
+                        L->maps, L->sd, pdl, d_label, 0, L->n_work);
                 QCK_CHECK_LAUNCH(h);
             }
         }

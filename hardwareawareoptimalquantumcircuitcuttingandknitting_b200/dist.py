@@ -165,10 +165,7 @@ _exchanges: dict = {}
 
 
 def stats_exchange(handle, device, group=None):
-    """The (cached) StatsExchange of this handle and group, or None when peer mailboxes are not available.
-    QCK_STATS_NCCL=1 keeps the NCCL path."""
-    if os.environ.get("QCK_STATS_NCCL", "0") == "1":
-        return None
+    """The (cached) StatsExchange of this handle and group, or None when peer mailboxes are not available."""
     key = (id(handle), str(device), id(group))
     ex = _exchanges.get(key)
     if ex is None:

@@ -190,10 +190,8 @@ class ContractCase:
 
 KERNEL_NAMES = {   # demangled kernel names as the CUDA profiler reports them
     "pipe128x16": "contract_dmma_pipe_kernel<128, 16>",
-    "pipe128x8": "contract_dmma_pipe_kernel<128, 8>",
     "pipe64": "contract_dmma_pipe_kernel<64, 8>",
     "dmma": "contract_dmma_kernel",
-    "fma": "contract_gemm_kernel",
     "generic": "contract_generic_kernel",
 }
 
@@ -245,15 +243,8 @@ CONTRACT_CASES = [
     _C("tile128_s7x7_65", (7, 7), ("cx", "cx", "cx"), "pipe128x16", env=(("QCK_CONTRACT_TILE", "128"),),
        labels=(17, 82)),
     _C("tile128_refused_s6x6", (6, 6), ("cx", "cx"), "pipe64", env=(("QCK_CONTRACT_TILE", "128"),)),
-    _C("warps8_s8x8_7776", (8, 8), ("cx",) * 5, "pipe128x8", env=(("QCK_CONTRACT_WARPS", "8"),)),
-    _C("warps8_s7x12_4096", (7, 12), ("wire",) * 4, "pipe128x8", touch=((0, 1, 2, 3), (2, 3)),
-       env=(("QCK_CONTRACT_WARPS", "8"),)),
-    _C("warps8_small_s6x6", (6, 6), ("cx", "cx"), "pipe64", env=(("QCK_CONTRACT_WARPS", "8"),)),
     _C("pipe0_s8x8_7776", (8, 8), ("cx",) * 5, "dmma", env=(("QCK_CONTRACT_PIPE", "0"),)),
     _C("pipe0_s7x7_65", (7, 7), ("cx", "cx", "cx"), "dmma", env=(("QCK_CONTRACT_PIPE", "0"),), labels=(17, 82)),
-    _C("fma_s8x8_7776", (8, 8), ("cx",) * 5, "fma", env=(("QCK_CONTRACT_FMA", "1"),)),
-    _C("fma_s1x9_hi", (1, 9), ("cx", "rzz"), "fma", layout="hi", env=(("QCK_CONTRACT_FMA", "1"),)),
-    _C("fma_s0x8", (0, 8), ("cx", "cx"), "fma", env=(("QCK_CONTRACT_FMA", "1"),)),
     _C("ctas1_s8x8_7776", (8, 8), ("cx",) * 5, "pipe128x16", env=(("QCK_CONTRACT_CTAS_PER_SM", "1"),)),
     _C("ctas8_s8x8_7776", (8, 8), ("cx",) * 5, "pipe128x16", env=(("QCK_CONTRACT_CTAS_PER_SM", "8"),)),
     _C("ctas64_s8x8_7776", (8, 8), ("cx",) * 5, "pipe128x16", env=(("QCK_CONTRACT_CTAS_PER_SM", "64"),)),
@@ -267,8 +258,6 @@ CONTRACT_CASES = [
        env=(("QCK_CONTRACT_CTAS_PER_SM", "1"),)),
     _C("ctas64_pipe0_s8x8_7776", (8, 8), ("cx",) * 5, "dmma",
        env=(("QCK_CONTRACT_CTAS_PER_SM", "64"), ("QCK_CONTRACT_PIPE", "0"))),
-    _C("ctas64_fma_s7x7_4097", (7, 7), ("cx",) * 5, "fma",
-       env=(("QCK_CONTRACT_CTAS_PER_SM", "64"), ("QCK_CONTRACT_FMA", "1")), labels=(0, 4097)),
     # ---- the generic kernel: masks that leave output bits uncovered, or three fragments without grouping
     _C("generic_uncovered", (3, 3), ("cx", "cx"), "generic", n_out=7),
     _C("generic_groups0_chain3", kernel="generic", env=(("QCK_CONTRACT_GROUPS", "0"),), **_CHAIN3),

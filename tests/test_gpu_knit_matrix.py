@@ -21,8 +21,8 @@ torch = pytest.importorskip("torch")
 from importlib import import_module  # noqa: E402
 
 _lib = import_module(f"{PKG}._lib")
-KNOBS = ("QCK_CONTRACT_TILE", "QCK_CONTRACT_WARPS", "QCK_CONTRACT_PIPE", "QCK_CONTRACT_FMA",
-         "QCK_CONTRACT_CTAS_PER_SM", "QCK_CONTRACT_GROUPS", "QCK_KO_CTAS_PER_SM")
+KNOBS = ("QCK_CONTRACT_TILE", "QCK_CONTRACT_PIPE", "QCK_CONTRACT_CTAS_PER_SM", "QCK_CONTRACT_GROUPS",
+         "QCK_KO_CTAS_PER_SM")
 
 
 @pytest.fixture(scope="module")
@@ -151,7 +151,7 @@ def test_contract_case(dev, clean_env, profiler_sees_kernels, name):
 
 
 SEQUENCE = ["s1x1", "s8x8_inter_7776", "s5x5_inter_15", "ctas64_s8x8_7776", "grouped_star4", "s8x8_32768", "count1",
-            "s10x10_4097_acc", "fma_s1x9_hi", "s7x12_4096", "ndigits0", "grouped_chain5", "s0x8"]
+            "s10x10_4097_acc", "s1x9_hi", "s7x12_4096", "ndigits0", "grouped_chain5", "s0x8"]
 
 
 def test_contract_sequence_without_sync(dev, clean_env):

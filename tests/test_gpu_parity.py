@@ -582,30 +582,25 @@ def _npd_async(dev, v, acc=0.0, shards=1):
     n_ws = h.lib.qck_npd_workspace_bytes() // 8
     if shards == 1:
         # at most 2^16 entries: ONE launch of one thread-block cluster (npd_cluster_kernel, the default); else - or
-        # with QCK_NPD_CLUSTER=0 - statistics + 6 level passes + apply, or one cooperative launch of the same
-        # passes (QCK_NPD_FUSED=1).  No host round trip in any form.  The staged and the cooperative form give the
-        # same bits; the cluster kernel finds the same partition and sums the dropped entries in another order.
+        # with QCK_NPD_CLUSTER=0 - statistics + 6 level passes + apply.  No host round trip in either form.  The
+        # cluster kernel finds the same partition as the staged one and sums the dropped entries in another order.
         import os
         results = {}
-        sms = torch.cuda.get_device_properties(dev).multi_processor_count
-        for form, env in (("cluster", {}), ("fused", {"QCK_NPD_CLUSTER": "0", "QCK_NPD_FUSED": "1"}),
-                          ("staged", {"QCK_NPD_CLUSTER": "0", "QCK_NPD_FUSED": "0"})):
+        for form, env in (("cluster", {}), ("staged", {"QCK_NPD_CLUSTER": "0"})):
             os.environ.update(env)
             try:
                 data = full.clone()
                 ws = torch.zeros(n_ws, dtype=torch.int64, device=dev)
                 l0 = h.launch_count
                 h.check(h.lib.qck_npd_async(h.ptr, data.data_ptr(), data.numel(), acc, ws.data_ptr(), stream))
-                one = (form == "cluster" and data.numel() <= 1 << 16) or \
-                      (form == "fused" and (data.numel() + 1023) // 1024 <= sms)
+                one = form == "cluster" and data.numel() <= 1 << 16
                 assert h.launch_count - l0 == (1 if one else 8), (form, h.launch_count - l0)
                 results[form] = (data.cpu().numpy(), ws[:32].cpu())
             finally:
                 for k in env:
                     os.environ.pop(k, None)
-        assert np.array_equal(results["fused"][0], results["staged"][0])
         a, b = results["cluster"], results["staged"]
-        assert int(a[1][5]) == int(b[1][5]) == int(results["fused"][1][5])
+        assert int(a[1][5]) == int(b[1][5])
         assert np.array_equal(a[0] == 0.0, b[0] == 0.0)                      # the same entries dropped
         assert np.abs(a[0] - b[0]).max() <= 4 * np.finfo(float).eps * max(1.0, np.abs(b[0]).max())
         assert a[1].view(torch.float64)[16] == b[1].view(torch.float64)[16]  # num: the number of survivors

@@ -1,5 +1,5 @@
 """Scratch: nearest_probability_distribution on the knitted 16-bit results of the BASELINE cuts - the one-cluster
-kernel (aggregation modes, per-phase cycle marks) against the staged launches.  CUDA events, median of 30."""
+kernel against the staged launches.  CUDA events, median of 30."""
 import os, sys
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
 import numpy as np
@@ -42,8 +42,6 @@ for wl in sys.argv[1:] or ["bv16", "hwe16d5", "syc16d5"]:
     print(f"{wl}: n={hv.size} neg={int((hv < 0).sum())} zero={int((hv == 0).sum())} min={hv.min():.3e} negsum={hv[hv < 0].sum():.3e}")
     t_ref, out_ref, st = timed(raw, {"QCK_NPD_CLUSTER": "0"})
     print(f"  staged (8 launches): {t_ref:.1f} us  status={st[5]} levels={st[18]}")
-    for mode in (0, 32):
-        t, out, st = timed(raw, {"QCK_NPC_MODE": str(mode | 64)})
-        marks = [int(x) for x in st[19:31] if x >= 0]
-        same = np.array_equal(out == 0, out_ref == 0) and np.abs(out - out_ref).max() < 1e-15
-        print(f"  cluster mode {mode}: {t:.1f} us  status={st[5]} levels={st[18]} same={same} marks(cycles)={marks}")
+    t, out, st = timed(raw, {})
+    same = np.array_equal(out == 0, out_ref == 0) and np.abs(out - out_ref).max() < 1e-15
+    print(f"  cluster (1 launch): {t:.1f} us  status={st[5]} levels={st[18]} same={same}")
