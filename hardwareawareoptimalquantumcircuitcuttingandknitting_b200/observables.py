@@ -23,12 +23,13 @@ Finite-shot estimates take sampled tables unchanged: with every fragment on ``B2
 from __future__ import annotations
 
 import ctypes as C
+from dataclasses import replace
 
 import numpy as np
 
 from . import _lib
 from .quasi_distr import default_device
-from .run import DenseResult, _all_b200, _finish_dense
+from .run import DenseResult, _all_b200, plan_step, post_step, read_step
 from .virtual_circuit import VirtualCircuit
 
 __all__ = ["expectation_values", "bitstring_probabilities", "marginal_distribution"]
@@ -177,5 +178,9 @@ def marginal_distribution(virt: VirtualCircuit, clbits, tables=None, device=None
         marg[f] = out
         kept_masks[f] = masks[f] & keep
     values = virt.knit_tables(marg, device, masks=kept_masks)
-    total, minimum = _finish_dense(handle, values, nearest, device, stream)
+    # the marginal's knit writes no statistics: npd or its statistics stage takes them, as with virtual gates
+    plan = replace(plan_step(virt), knit_stats=False)
+    ws = handle.npd_workspace(torch, device)
+    post_step(handle, plan, values, ws, None, nearest, stream=stream)
+    total, minimum = read_step(plan, ws, None, None, nearest)
     return DenseResult(values, keep, total, minimum)

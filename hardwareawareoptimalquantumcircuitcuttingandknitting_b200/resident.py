@@ -9,7 +9,10 @@ all-reduce of a multi-rank run, the statistics and the threshold search of npd -
 free of host round trips, so it can be captured once (``torch.cuda.graph``) and replayed with a single
 launch.  ``run_virtual_circuit_dense`` stays the eager entry point (a new circuit every call: nothing to
 replay); this class serves repeated evaluation of one cut circuit (the reference runs every cut circuit
-at least twice, ``Utilities.py:85-86``) and ``bench.py``'s resident ``value``.
+at least twice, ``Utilities.py:85-86``) and ``bench.py``'s resident ``value``.  Both run the same step: the
+decisions of ``run.plan_step``, carried out by ``run.knit_step``, ``run.post_step`` and ``run.read_step``.  Only the
+eager call, which reads the statistics back before it decides, runs npd on a K = 0 exact result (when its
+minimum is negative); a resident K = 0 exact step never does.
 
 Buffers (fragment tables, result, statistics, npd workspace) are allocated once and reused by every step:
 ``result()`` reads the state of the LAST step.
@@ -18,7 +21,7 @@ from __future__ import annotations
 
 from . import _lib
 from .quasi_distr import default_device
-from .run import DenseResult, _check_npd_state
+from .run import DenseResult, knit_step, plan_step, post_step, read_step
 from .virtual_circuit import VirtualCircuit
 
 __all__ = ["ResidentStep"]
@@ -36,42 +39,24 @@ class ResidentStep:
         if virt.noisy_fragments():
             raise NotImplementedError("ResidentStep runs state-vector fragment programs; a fragment is bound to a "
                                       "noisy B200Backend (use run_virtual_circuit or run_virtual_circuit_dense)")
-        self.torch, self.qdist = torch, qdist
         self.virt = virt
-        self.device = default_device() if device is None else torch.device(device)
-        self.handle = _lib.get_handle(self.device.index or 0)
-        self.nearest, self.rank, self.world, self.group = nearest, rank, world_size, group
-        self.accuracy = float(accuracy)
-        self.faithful = self.accuracy > 0.0
-        self.K = len(virt.vgates)
-        masks, self.union = virt.output_masks()
-        self.n_out = bin(self.union).count("1")
-        self.frags = virt.active_fragments()
-        L = virt.num_global_labels()
-        self.mode = "single"
-        if world_size > 1:
-            self.mode = ("output index by top bits" if self.K == 0
-                         else qdist.partition_mode(virt, world_size, self.faithful))
-        self.label_range = None
-        self.entry_sharded = self.mode == "output entries + all-reduce" and self.K > 0
-        if self.K == 0:
-            self.y0, self.y1 = (qdist.shard_pow2(self.n_out, rank, world_size) if world_size > 1
-                                else (0, 1 << self.n_out))
-        else:
-            self.y0, self.y1 = 0, 1 << self.n_out
-            if self.mode == "label range + all-reduce":
-                self.label_range = qdist.shard_range(L, rank, world_size, align=virt.global_radices()[-1])
-        dev = self.device
+        self.device = dev = default_device() if device is None else torch.device(device)
+        self.handle = _lib.get_handle(dev.index or 0)
+        self.nearest, self.group = nearest, group
+        self.plan = plan = plan_step(virt, rank, world_size, float(accuracy))
+        self.mode, self.label_range = plan.mode, plan.label_range
+        self.y0, self.y1 = plan.y_range if plan.y_range is not None else (0, 1 << plan.n_out)
         self.out = out if out is not None else torch.empty(self.y1 - self.y0, dtype=torch.float64, device=dev)
         self.stats = torch.zeros(4, dtype=torch.float64, device=dev)
         self.ws = self.handle.npd_workspace(torch, dev)
-        self.execs, self.tables = [], {}
-        for f in self.frags:
-            ex = virt.executor(f, dev, not self.faithful)
+        self.exchange = (qdist.stats_exchange(self.handle, self.stats.device, group)
+                         if plan.collective == "allreduce_stats" else None)
+        self.tables = {}
+        for f in virt.active_fragments():
+            ex = virt.executor(f, dev, plan.fold)
             ex.upload()
-            alloc = torch.zeros if self.label_range is not None else torch.empty
+            alloc = torch.zeros if plan.label_range is not None else torch.empty
             self.tables[f] = alloc((ex.program.num_labels, ex.row_len), dtype=torch.float64, device=dev)
-            self.execs.append(ex)
         self._graph = None
         self._graph_body = None
         self._phase_graphs = None
@@ -79,46 +64,17 @@ class ResidentStep:
 
     # ---------------------------------------------------------------- the three phases of a step
     def enqueue_simulation(self) -> None:
-        virt = self.virt
-        virt.simulate_fragments(self.device, label_range=self.label_range, fold=not self.faithful, out=self.tables)
+        self.virt.simulate_fragments(self.device, label_range=self.plan.label_range, fold=self.plan.fold,
+                                     out=self.tables)
 
     def enqueue_knit(self) -> None:
-        virt, dev = self.virt, self.device
-        if self.faithful:
-            virt.knit_tables_faithful(self.tables, self.accuracy, dev, out=self.out,
-                                      part=(self.rank, self.world) if self.entry_sharded else (0, 1))
-        elif self.K == 0:
-            virt.knit_tables(self.tables, dev, stats=self.stats,
-                             y_range=(self.y0, self.y1) if self.world > 1 else None, out=self.out,
-                             exchange=self._exchange())
-        else:
-            virt.knit_tables(self.tables, dev, label_range=self.label_range, out=self.out)
+        knit_step(self.virt, self.plan, self.tables, self.device, self.out, self.stats, self.exchange)
 
     def enqueue_post(self) -> None:
         """Collectives, statistics and nearest_probability_distribution (``run.py:71``)."""
-        torch = self.torch
-        stream = torch.cuda.current_stream(self.device).cuda_stream
-        h = self.handle
-        if self.K == 0:
-            if self.world > 1 and self._exchange() is None:     # (else exchanged in the knit kernel's tail)
-                self.qdist.allreduce_stats(self.stats, self.group, self.handle)   # min >= 0: no npd pass
-            return
-        if self.label_range is not None or self.entry_sharded:
-            self.qdist.allreduce_sum_(self.out, self.group)
-        if self.nearest:
-            h.check(h.lib.qck_npd_async(h.ptr, self.out.data_ptr(), self.out.numel(), self.accuracy,
-                                        self.ws.data_ptr(), stream))
-        else:
-            h.check(h.lib.qck_npd_stage(h.ptr, _lib.NPD_STATS, self.out.data_ptr(), self.out.numel(), self.accuracy,
-                                        self.ws.data_ptr(), 1, stream))
-
-    def _exchange(self):
-        """Peer mailboxes of a result sharded by output index (K = 0, world > 1), or None (NCCL path)."""
-        if self.world <= 1 or self.K != 0 or self.faithful:
-            return None
-        if not hasattr(self, "_ex"):
-            self._ex = self.qdist.stats_exchange(self.handle, self.device, self.group)
-        return self._ex
+        import torch
+        post_step(self.handle, self.plan, self.out, self.ws, self.stats, self.nearest, self.group,
+                  torch.cuda.current_stream(self.device).cuda_stream)
 
     def enqueue(self) -> None:
         self.enqueue_simulation()
@@ -129,7 +85,7 @@ class ResidentStep:
     def capture(self, phases: bool = False):
         """Warm up eagerly (scratch buffers, side streams, function attributes - nothing may allocate during
         the capture), then capture the step - or, with ``phases``, its three phases as separate graphs."""
-        torch = self.torch
+        import torch
         side = torch.cuda.Stream(self.device)
         side.wait_stream(torch.cuda.current_stream(self.device))
         with torch.cuda.stream(side):
@@ -141,9 +97,8 @@ class ResidentStep:
         # collectives with the communicator, and tearing the graph down later (its private memory pool goes with
         # it) left a 2-rank run with an illegal memory access in the next eager collective.  The collective and
         # what follows it are a handful of launches; they stay eager.
-        mailboxes = self.world > 1 and self.K == 0 and self.qdist.stats_exchange(self.handle, self.device, self.group)
-        post_has_collective = self.world > 1 and ((self.K == 0 and not mailboxes) or self.label_range is not None
-                                                  or self.entry_sharded)
+        post_has_collective = (self.plan.collective == "allreduce_sum"
+                               or (self.plan.collective == "allreduce_stats" and self.exchange is None))
 
         class _Eager:                                  # same interface as a CUDAGraph
             def __init__(self, fn):
@@ -183,10 +138,5 @@ class ResidentStep:
 
     def result(self) -> DenseResult:
         """Statistics of the last step (one small device -> host read; synchronises)."""
-        if self.K == 0:
-            host = self.stats.cpu().numpy()
-            total, minimum = float(host[0]), float(host[1])
-        else:
-            state = _check_npd_state(self.ws, solved=self.nearest)
-            total, minimum = float(state[0]), float(state[1])
-        return DenseResult(self.out, self.union, total, minimum, self.y0)
+        total, minimum = read_step(self.plan, self.ws, self.stats, None, self.nearest)
+        return DenseResult(self.out, self.plan.union, total, minimum, self.y0)

@@ -20,6 +20,11 @@ If a fragment is bound to a foreign duck-typed backend
 circuits, the backend's counts, ``QuasiDistr.from_counts`` and the
 reference-order ``virt.knit`` - still on device-resident distributions.
 
+A dense step's decisions - the labels this rank simulates, the output slice it owns, the knit and the collective
+that run, where ``total`` and ``minimum`` come from - are made once by ``plan_step``.  ``knit_step``, ``post_step``
+and ``read_step`` carry them out for ``run_virtual_circuit_dense``, for the foreign-backend path and for
+``resident.ResidentStep``, which replays them as a CUDA graph.
+
 The four log lines of the reference (``run.py:28-32,45,62,69``) are kept, through
 the standard ``logging`` module.
 """
@@ -33,6 +38,7 @@ from time import perf_counter
 import numpy as np
 
 from . import _lib
+from . import dist as qdist
 from .backend import B200Backend
 from .quasi_distr import default_device
 from .virtual_circuit import VirtualCircuit, generate_instantiations
@@ -85,16 +91,147 @@ def _all_b200(virt: VirtualCircuit) -> bool:
     return all(isinstance(virt.get_backend(f), B200Backend) for f in virt.fragment_circuits)
 
 
+@dataclass(frozen=True)
+class StepPlan:
+    """Every decision of one dense step, made once by ``plan_step``.
+
+    ``faithful``: ``accuracy > 0``, the reference-faithful knit of unfolded tables (``fold`` False).  ``union`` /
+    ``n_out``: the written clbits and their number.  ``mode``: how the ranks share the step.  ``label_range``: the
+    global labels this rank simulates and knits (None: all).  ``y_range``: the output slice this rank owns (None: the
+    whole vector).  ``part``: this rank's share of the faithful knit's output entries.  ``collective``: what follows
+    the knit across ranks - "allreduce_stats" (the K = 0 statistics; peer mailboxes do it in the knit kernel's
+    tail), "allreduce_sum" (the dense result) or None.  ``knit_stats``: the knit writes ``total`` / ``minimum``
+    itself (K = 0, exact); otherwise they come from the npd state."""
+    K: int
+    faithful: bool
+    fold: bool
+    union: int
+    n_out: int
+    mode: str
+    label_range: tuple[int, int] | None
+    y_range: tuple[int, int] | None
+    part: tuple[int, int]
+    collective: str | None
+    knit_stats: bool
+    accuracy: float
+
+
+def plan_step(virt: VirtualCircuit, rank: int = 0, world_size: int = 1, accuracy: float = 0.0) -> StepPlan:
+    """The decisions of a dense step on ``rank`` of ``world_size`` (``dist.py``): without virtual gates the output
+    index is sharded by its top bits; with them the labels are sharded above ``dist.SHARD_MIN_WORK`` (else every
+    rank computes everything); the faithful knit shares its output entries instead, and runs replicated without
+    virtual gates."""
+    K = len(virt.vgates)
+    faithful = accuracy > 0.0
+    _, union = virt.output_masks()
+    n_out = bin(union).count("1")
+    if world_size <= 1:
+        mode = "single"
+    elif K == 0:
+        mode = "replicated" if faithful else "output index by top bits"
+    else:
+        mode = qdist.partition_mode(virt, world_size, faithful)
+    label_range = (qdist.shard_range(virt.num_global_labels(), rank, world_size, align=virt.global_radices()[-1])
+                   if mode == "label range + all-reduce" else None)
+    y_range = qdist.shard_pow2(n_out, rank, world_size) if mode == "output index by top bits" else None
+    part = (rank, world_size) if mode == "output entries + all-reduce" else (0, 1)
+    collective = ("allreduce_stats" if y_range is not None else
+                  "allreduce_sum" if label_range is not None or part != (0, 1) else None)
+    return StepPlan(K, faithful, not faithful, union, n_out, mode, label_range, y_range, part, collective,
+                    K == 0 and not faithful, float(accuracy) if faithful else 0.0)
+
+
+def knit_step(virt: VirtualCircuit, plan: StepPlan, tables: dict, device, out=None, stats=None, exchange=None):
+    """The step's knit: the reference-faithful knit, ``knit_outer`` (K = 0: it also writes ``stats``, combined
+    across the ranks in its tail when ``exchange`` holds peer mailboxes) or ``knit_contract`` (K > 0)."""
+    if plan.faithful:
+        return virt.knit_tables_faithful(tables, plan.accuracy, device, out=out, part=plan.part)
+    if plan.K == 0:
+        return virt.knit_tables(tables, device, stats=stats, y_range=plan.y_range, out=out, exchange=exchange)
+    return virt.knit_tables(tables, device, label_range=plan.label_range, out=out)
+
+
+def post_step(handle, plan: StepPlan, values, ws, stats, nearest: bool, group=None, stream: int = 0) -> None:
+    """What follows the knit, enqueued without a host read (a graph can capture it): the collective, then
+    ``nearest_probability_distribution`` (``nearest``) or its statistics stage alone, at the plan's accuracy.  With
+    ``knit_stats`` the knit has written the statistics and nothing more is enqueued."""
+    if plan.collective == "allreduce_stats":
+        if qdist.stats_exchange(handle, stats.device, group) is None:    # (else exchanged in the knit's tail)
+            qdist.allreduce_stats(stats, group)
+    elif plan.collective == "allreduce_sum":
+        qdist.allreduce_sum_(values, group)
+    if plan.knit_stats:
+        return
+    if nearest:
+        handle.check(handle.lib.qck_npd_async(handle.ptr, values.data_ptr(), values.numel(), plan.accuracy,
+                                              ws.data_ptr(), stream))
+    else:
+        handle.check(handle.lib.qck_npd_stage(handle.ptr, _lib.NPD_STATS, values.data_ptr(), values.numel(),
+                                              plan.accuracy, ws.data_ptr(), 1, stream))
+
+
+def read_step(plan: StepPlan, ws, stats, status=None, nearest: bool = True) -> tuple[float, float]:
+    """(total, minimum) of the knitted quasi-distribution: the step's one device -> host read (synchronises), from
+    ``stats`` with ``knit_stats``, else from the npd state in ``ws``.  ``status``: the sampler's status word, read
+    in the same copy (raises when it is set).  After npd the state is checked (``_check_npd_state``)."""
+    import torch
+    src = stats if plan.knit_stats else ws[:_lib.NPD_STATE_SLOTS]
+    if status is not None:
+        src = torch.cat([src.view(torch.int64), status])
+    host = src.cpu().numpy().view(np.int64)
+    if status is not None:
+        from .sampling import raise_for_status
+        raise_for_status(int(host[-1]))
+    if nearest and not plan.knit_stats:
+        _check_npd_state(host)
+    total, minimum = host[:2].view(np.float64).tolist()
+    return total, minimum
+
+
+def _check_npd_state(state) -> None:
+    """Raises where the reference would fail (negative total: quasi_distr.py:36 ends in a division by zero) or
+    where the threshold search of qck_npd_async / npd_sharded did not finish.  ``state``: the workspace's first
+    NPD_STATE_SLOTS slots, read back as int64 numpy."""
+    status = int(state[5])
+    if status == _lib.NPD_ST_NEGATIVE_TOTAL:
+        total = state[:1].view(np.float64)[0]
+        raise ValueError(f"nearest_probability_distribution: total mass {total:.3e} is negative")
+    if status not in (_lib.NPD_ST_IDENTITY, _lib.NPD_ST_SOLVED):
+        raise RuntimeError(f"nearest_probability_distribution: threshold search did not finish (status {status})")
+
+
+def _knit_eager(virt, plan: StepPlan, tables: dict, device, handle, nearest: bool, out=None, group=None,
+                status=None) -> tuple:
+    """knit_step, post_step and read_step, launched as they come -> (values, total, minimum).  K = 0, exact: a
+    product of fragment probabilities, so npd runs only when the read-back minimum is negative."""
+    import torch
+    stream = torch.cuda.current_stream(device).cuda_stream
+    ws = handle.npd_workspace(torch, device)
+    stats = torch.zeros(4, dtype=torch.float64, device=device) if plan.knit_stats else None
+    exchange = (qdist.stats_exchange(handle, stats.device, group) if plan.collective == "allreduce_stats"
+                else None)
+    values = knit_step(virt, plan, tables, device, out, stats, exchange)
+    post_step(handle, plan, values, ws, stats, nearest, group, stream)
+    total, minimum = read_step(plan, ws, stats, status, nearest)
+    if plan.knit_stats and nearest and minimum < 0.0:
+        if plan.y_range is not None:
+            qdist.npd_sharded(handle, values, 0.0, ws, group, stream)
+        else:
+            handle.check(handle.lib.qck_npd_async(handle.ptr, values.data_ptr(), values.numel(), 0.0,
+                                                  ws.data_ptr(), stream))
+        _check_npd_state(ws[:_lib.NPD_STATE_SLOTS].cpu().numpy())
+    return values, total, minimum
+
+
 def run_virtual_circuit_dense(virt: VirtualCircuit, shots: int = 20000, device=None, nearest: bool = True,
                               rank: int = 0, world_size: int = 1, group=None,
                               out=None, accuracy: float | None = None) -> tuple[DenseResult, RunTimeInfo]:
     """Whole path on the GPU.  With ``world_size > 1`` (one process per GPU) the work is
-    partitioned as described in ``dist.py``: without virtual gates this rank produces the
+    partitioned as described in ``dist.py`` and ``plan_step``: without virtual gates this rank produces the
     output slice whose top bits equal ``rank`` (``DenseResult.y_begin`` tells where it
     starts); with virtual gates the labels are sharded and the dense result is all-reduced,
-    so every rank returns the full vector."""
+    so every rank returns the full vector.  ``accuracy`` None: ``quasi_distr.ACCURACY``."""
     import torch
-    from . import dist as qdist
     if not _all_b200(virt):
         raise ValueError("run_virtual_circuit_dense needs every fragment on a B200Backend")
     device = default_device() if device is None else torch.device(device)
@@ -103,60 +240,25 @@ def run_virtual_circuit_dense(virt: VirtualCircuit, shots: int = 20000, device=N
     logger.info(f"Running virtualizer with {len(frags)} "
                 + f"{tuple(circ.num_qubits for circ in frags.values())} "
                 + f"fragments and {len(virt._vgate_instrs)} vgates...")
-    K = len(virt._vgate_instrs)
     from . import quasi_distr as _qd
-    accuracy = _qd.ACCURACY if accuracy is None else float(accuracy)
+    plan = plan_step(virt, rank, world_size, _qd.ACCURACY if accuracy is None else float(accuracy))
     sample_shots = _sample_shots(virt, shots, world_size)
-    if accuracy > 0.0:
-        return _run_faithful(virt, device, handle, nearest, accuracy, rank, world_size, group, out, sample_shots)
-    label_range = None
-    if K > 0 and world_size > 1 and qdist.partition_mode(virt, world_size) == "label range + all-reduce":
-        label_range = qdist.shard_range(virt.num_global_labels(), rank, world_size,
-                                        align=virt.global_radices()[-1])
-    stream = torch.cuda.current_stream(device).cuda_stream
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
     ev[0].record()
     logger.info(f"Running {sum(virt.program(f).num_labels for f in virt.active_fragments())} instances...")
-    tables = virt.simulate_fragments(device, label_range=label_range, shots=sample_shots)
+    tables = virt.simulate_fragments(device, label_range=plan.label_range, fold=plan.fold, shots=sample_shots)
     status = virt.sample_status if sample_shots is not None else None
     ev[1].record()
 
     logger.info("Knitting...")
-    _, union = virt.output_masks()
-    y_begin = 0
-    ws = None
-    if K == 0:
-        # products of fragment probabilities: the minimum comes with the knit's own statistics, so the
-        # 2^n_out-entry result is only read again when it really has negative entries
-        stats = torch.zeros(4, dtype=torch.float64, device=device)
-        n_out = bin(union).count("1")
-        y_range = qdist.shard_pow2(n_out, rank, world_size) if world_size > 1 else None
-        y_begin = y_range[0] if y_range else 0
-        ex = qdist.stats_exchange(handle, device, group) if world_size > 1 else None
-        values = virt.knit_tables(tables, device, stats=stats, y_range=y_range, out=out, exchange=ex)
-        if ex is None:                            # (else the knit kernel's tail has exchanged them already)
-            qdist.allreduce_stats(stats, group, handle)
-        host_stats = _read_back(stats, status)    # the step's device -> host read (synchronises)
-        total, minimum = float(host_stats[0]), float(host_stats[1])
-        if nearest and minimum < 0.0:
-            ws = handle.npd_workspace(torch, device)
-            if world_size > 1:
-                qdist.npd_sharded(handle, values, 0.0, ws, group, stream)
-            else:
-                handle.check(handle.lib.qck_npd_async(handle.ptr, values.data_ptr(), values.numel(), 0.0,
-                                                      ws.data_ptr(), stream))
-            _check_npd_state(ws)
-    else:
-        values = virt.knit_tables(tables, device, label_range=label_range, out=out)
-        if label_range is not None:
-            qdist.allreduce_sum_(values, group)
-        total, minimum = _finish_dense(handle, values, nearest, device, stream, status)
+    values, total, minimum = _knit_eager(virt, plan, tables, device, handle, nearest, out, group, status)
     ev[2].record()
     ev[2].synchronize()
     # device time of the two phases (run.py:60,67 take wall-clock times around the same two phases)
     run_time, knit_time = ev[0].elapsed_time(ev[1]) * 1e-3, ev[1].elapsed_time(ev[2]) * 1e-3
     logger.info(f"Knitted in {knit_time:.2f}s.")
-    return DenseResult(values, union, total, minimum, y_begin), RunTimeInfo(run_time, knit_time)
+    y_begin = plan.y_range[0] if plan.y_range is not None else 0
+    return DenseResult(values, plan.union, total, minimum, y_begin), RunTimeInfo(run_time, knit_time)
 
 
 def _sample_shots(virt: VirtualCircuit, shots: int, world_size: int) -> int | None:
@@ -168,94 +270,6 @@ def _sample_shots(virt: VirtualCircuit, shots: int, world_size: int) -> int | No
         raise ValueError("a sampled multi-rank run needs B200Backend(sampling=True, seed=<int>): every rank must "
                          "draw the same counts")
     return int(shots)
-
-
-def _read_back(stats, status=None):
-    """stats (float64 device vector) -> host numpy; with the sampler's status word appended in the same copy
-    (raises when it is set)."""
-    import torch
-    if status is None:
-        return stats.cpu().numpy()
-    host = torch.cat([stats.view(torch.int64), status]).cpu()
-    from .sampling import raise_for_status
-    raise_for_status(int(host[-1]))
-    return host[:-1].view(torch.float64).numpy()
-
-
-def _finish_dense(handle, values, nearest: bool, device, stream, status=None) -> tuple[float, float]:
-    """Total and minimum of a knitted dense quasi-distribution (synchronises); with ``nearest`` it is
-    then replaced in place by ``nearest_probability_distribution``.  ``status``: the sampler's status word,
-    read back with the statistics."""
-    import torch
-    if nearest:
-        # statistics, threshold search and shift are all enqueued (qck_npd_async: no host round
-        # trip); the statistics of the knitted quasi-distribution come back with its state
-        ws = handle.npd_workspace(torch, device)
-        handle.check(handle.lib.qck_npd_async(handle.ptr, values.data_ptr(), values.numel(), 0.0,
-                                              ws.data_ptr(), stream))
-        state = _check_npd_state(ws, status=status)   # the step's device -> host read (synchronises)
-        return float(state[0]), float(state[1])
-    stats = torch.zeros(4, dtype=torch.float64, device=device)
-    handle.check(handle.lib.qck_stats_dense(handle.ptr, values.data_ptr(), values.numel(), 0.0,
-                                            stats.data_ptr(), stream))
-    host_stats = _read_back(stats, status)
-    return float(host_stats[0]), float(host_stats[1])
-
-
-def _check_npd_state(ws, solved: bool = True, status=None):
-    """Reads the 256-byte state qck_npd_async / npd_sharded left in the workspace (synchronises) and
-    raises where the reference would fail (negative total: quasi_distr.py:36 ends in a division by zero).
-    ``status``: the sampler's status word, read in the same copy."""
-    import torch
-    if status is not None:
-        host = torch.cat([ws[:_lib.NPD_STATE_SLOTS], status]).cpu()
-        from .sampling import raise_for_status
-        raise_for_status(int(host[-1]))
-        state = host[:-1]
-    else:
-        state = ws[:_lib.NPD_STATE_SLOTS].cpu()
-    status = int(state[5])
-    state = state.view(torch.float64).numpy()
-    if solved and status == _lib.NPD_ST_NEGATIVE_TOTAL:
-        raise ValueError(f"nearest_probability_distribution: total mass {state[0]:.3e} is negative")
-    if solved and status not in (_lib.NPD_ST_IDENTITY, _lib.NPD_ST_SOLVED):
-        raise RuntimeError(f"nearest_probability_distribution: threshold search did not finish (status {status})")
-    return state
-
-
-def _run_faithful(virt, device, handle, nearest, accuracy, rank, world_size, group, out, shots=None):
-    """ACCURACY > 0: exact instance distributions, then the reference's pruned algebra in the
-    reference's order, fused per output entry (``qck_knit_faithful``).  Every output entry is an
-    independent expression tree: with ``world_size > 1`` every rank simulates the (small) fragments itself,
-    evaluates its share of the output entries and the shares are added up with one all-reduce."""
-    import torch
-    from . import dist as qdist
-    stream = torch.cuda.current_stream(device).cuda_stream
-    ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
-    ev[0].record()
-    tables = virt.simulate_fragments(device, fold=False, shots=shots)
-    status = virt.sample_status if shots is not None else None
-    ev[1].record()
-    logger.info("Knitting...")
-    sharded = world_size > 1 and len(virt._vgate_instrs) > 0
-    values = virt.knit_tables_faithful(tables, accuracy, device, out=out, part=(rank, world_size) if sharded else (0, 1))
-    if sharded:
-        qdist.allreduce_sum_(values, group)
-    ws = handle.npd_workspace(torch, device)
-    if nearest:
-        handle.check(handle.lib.qck_npd_async(handle.ptr, values.data_ptr(), values.numel(), accuracy,
-                                              ws.data_ptr(), stream))
-    else:
-        handle.check(handle.lib.qck_npd_stage(handle.ptr, _lib.NPD_STATS, values.data_ptr(), values.numel(),
-                                              accuracy, ws.data_ptr(), 1, stream))
-    state = _check_npd_state(ws, solved=nearest, status=status)
-    total, minimum = float(state[0]), float(state[1])
-    ev[2].record()
-    ev[2].synchronize()
-    run_time, knit_time = ev[0].elapsed_time(ev[1]) * 1e-3, ev[1].elapsed_time(ev[2]) * 1e-3
-    logger.info(f"Knitted in {knit_time:.2f}s.")
-    _, union = virt.output_masks()
-    return DenseResult(values, union, total, minimum, 0), RunTimeInfo(run_time, knit_time)
 
 
 def _experiment_counts(result, n: int):
@@ -342,8 +356,8 @@ def run_virtual_circuit(virt: VirtualCircuit, shots: int = 20000) -> tuple[dict[
     from . import quasi_distr as _qd
     device = default_device()
     handle = _lib.get_handle(device.index or 0)
-    accuracy = float(_qd.ACCURACY)
-    fold = accuracy <= 0.0
+    plan = plan_step(virt, 0, 1, float(_qd.ACCURACY))
+    fold = plan.fold
     jobs, tables = {}, {}
     from .sampling import new_status
     status = None
@@ -380,16 +394,8 @@ def run_virtual_circuit(virt: VirtualCircuit, shots: int = 20000) -> tuple[dict[
     run_time = perf_counter() - now
     logger.info("Knitting...")
     now = perf_counter()
-    stream = torch.cuda.current_stream(device).cuda_stream
-    if fold:
-        values = virt.knit_tables(tables, device)
-    else:
-        values = virt.knit_tables_faithful(tables, accuracy, device)
-    ws = handle.npd_workspace(torch, device)
-    handle.check(handle.lib.qck_npd_async(handle.ptr, values.data_ptr(), values.numel(), accuracy, ws.data_ptr(),
-                                          stream))
-    state = _check_npd_state(ws, status=status)
+    values, total, minimum = _knit_eager(virt, plan, tables, device, handle, True, status=status)
     knit_time = perf_counter() - now
     logger.info(f"Knitted in {knit_time:.2f}s.")
     _, union = virt.output_masks(list(tables))
-    return DenseResult(values, union, float(state[0]), float(state[1]), 0).to_dict(), RunTimeInfo(run_time, knit_time)
+    return DenseResult(values, union, total, minimum, 0).to_dict(), RunTimeInfo(run_time, knit_time)

@@ -79,7 +79,7 @@ def main() -> None:
         h = lib.get_handle(local_rank)
         ws = h.npd_workspace(torch, dev)
         qdist.npd_sharded(h, mine, 0.0, ws, None, torch.cuda.current_stream(dev).cuda_stream)
-        state = runm._check_npd_state(ws)
+        runm._check_npd_state(ws[:lib.NPD_STATE_SLOTS].cpu().numpy())
         err = float(np.abs(mine.cpu().numpy() - want[lo:hi]).max())
         assert err < 1e-13, (make, rank, err)
         worst = max(worst, err)
@@ -135,9 +135,10 @@ def main() -> None:
     del rs, eager
 
     # (6) reference-default mode (ACCURACY = 1e-5): every rank evaluates its share of the output entries, one
-    #     all-reduce adds the shares - the same BITS as the one-GPU evaluation, eagerly and as a resident step
-    for cfg in ("syc16d5", "hwe16d5"):
-        circ, cut = cutting.make_baseline(cfg, seed=1)
+    #     all-reduce adds the shares - the same BITS as the one-GPU evaluation, eagerly and as a resident step.
+    #     Without virtual gates (syc-20) every rank knits the whole output itself.
+    cases = [(cfg,) + cutting.make_baseline(cfg, seed=1) for cfg in ("syc16d5", "hwe16d5")] + [("syc20", c20, cut20)]
+    for cfg, circ, cut in cases:
         assert qdist.partition_mode(vcm.VirtualCircuit(cut), world, faithful=True) == "output entries + all-reduce"
         one, _ = runm.run_virtual_circuit_dense(vcm.VirtualCircuit(cut), device=dev, nearest=False, accuracy=1e-5)
         many, _ = runm.run_virtual_circuit_dense(vcm.VirtualCircuit(cut), device=dev, nearest=False, accuracy=1e-5,
@@ -147,7 +148,9 @@ def main() -> None:
                                accuracy=1e-5, graph=True)
         for _ in range(2):
             rs.run()
-        assert torch.equal(rs.result().values, one.values), (cfg, rank)
+        got = rs.result()
+        assert torch.equal(got.values, one.values), (cfg, rank)
+        assert (got.total, got.minimum) == (one.total, one.minimum) == (many.total, many.minimum), (cfg, rank)
         uncut = cport.simulate_probabilities(circ)
         assert float(np.abs(many.values.cpu().numpy() - uncut).max()) < 7776 * 1e-5      # within the pruning error
         dist.barrier()

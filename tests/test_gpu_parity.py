@@ -1299,3 +1299,20 @@ def test_resident_step_graph_replay(dev, cfg):
     rs.out.zero_()
     g_sim.replay(); g_knit.replay(); g_post.replay()
     assert torch.equal(rs.result().values, ref_vals)
+
+
+def test_resident_step_faithful_without_virtual_gates(dev):
+    """ResidentStep at ACCURACY = 1e-5 on a cut without virtual gates runs the eager call's step: the faithful knit of
+    the whole output, npd at that accuracy, total and minimum from the npd state - eagerly and as graph replays."""
+    resm = import_module(f"{PKG}.resident")
+    c = gen.gen_circ("syc", 20, 1, seed=0).decompose_two_qubit()
+    cut = cutting.apply_cuts(c, cutting.CutSpec(partitions=[list(range(10)), list(range(10, 20))]))
+    want, _ = runm.run_virtual_circuit_dense(vcm.VirtualCircuit(cut), device=dev, accuracy=1e-5)
+    assert want.values.numel() == 1 << 20 and want.total > 0.5
+    for graph in (False, True):
+        rs = resm.ResidentStep(vcm.VirtualCircuit(cut), dev, accuracy=1e-5, graph=graph)
+        for _ in range(3):
+            rs.run()
+        got = rs.result()
+        assert torch.equal(got.values, want.values), graph
+        assert got.total == want.total and got.minimum == want.minimum, (graph, got.total, want.total)
