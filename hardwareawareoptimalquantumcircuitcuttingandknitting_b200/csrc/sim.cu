@@ -1502,6 +1502,16 @@ static int warp_group_layout(qck_handle* h, const qck_sim_plan* plans, const int
             p.sweeps[0].op_end - p.sweeps[0].op_begin > 60000)
             QCK_FAIL(h, QCK_ERR_INVALID_ARG, "register-resident plan out of range (%d qubits, %d branch points)",
                      G.n_base, n_anc);
+        // the leaves are signed by every sign_mask bit and all of them are added: a sign on an unsummed bit, or an
+        // outcome bit that is neither a row bit nor summed, would give other rows than the shared-memory kernels
+        unsigned long long row_bits = 0;
+        for (int j = 0; j < p.n_out_bits; ++j)
+            if (p.out_pos[j] >= 0) row_bits |= 1ull << p.out_pos[j];
+        if (p.sign_mask & ~p.sum_mask)
+            QCK_FAIL(h, QCK_ERR_INVALID_ARG, "register-resident plan: sign_mask bits outside sum_mask");
+        for (int a = G.n_base; a < p.n_state_qubits; ++a)
+            if (!(((p.sum_mask | row_bits) >> a) & 1ull))
+                QCK_FAIL(h, QCK_ERR_INVALID_ARG, "register-resident plan: outcome bit %d is neither a row bit nor summed", a);
         WarpVarDev& v = G.var[i];
         v.op_begin = p.sweeps[0].op_begin;
         v.op_end = p.sweeps[0].op_end;
@@ -1706,6 +1716,26 @@ extern "C" int qck_sim_tree(qck_handle* h, const qck_sim_tree_plan* plan, int64_
         if (L.qubit < 0 || L.qubit >= plan->n_base || (L.kind != QCK_TREE_MMEAS && (L.digit < 0 || L.digit >= plan->n_digits)))
             QCK_FAIL(h, QCK_ERR_INVALID_ARG, "tree level %d: bad qubit / digit", l);
     }
+    // refusals of the combine: checked before anything is launched
+    int n_fork_max = 0;
+    long long n_rep_labels = 1, n_eq_max = 1;
+    for (int l = 0; l < plan->n_levels; ++l) {
+        const qck_tree_level& L = plan->level[l];
+        if (L.kind == QCK_TREE_MMEAS) continue;
+        n_fork_max += L.kind == QCK_TREE_SLOT;
+        int reps = 0, biggest = 1;
+        for (int v = 0; v < 8; ++v) {
+            if (L.first_choice[v] < 0) continue;
+            ++reps;
+            int cls = 0;
+            for (int d = 0; d < plan->radix[L.digit]; ++d) cls += (int)((L.canon >> (4 * d)) & 15u) == v;
+            if (cls > biggest) biggest = cls;
+        }
+        n_rep_labels *= reps;
+        n_eq_max *= biggest;
+    }
+    if (n_fork_max > 8) QCK_FAIL(h, QCK_ERR_UNSUPPORTED, "more than 8 measuring slots whose qubit lives on");
+    if (n_eq_max > 256) QCK_FAIL(h, QCK_ERR_UNSUPPORTED, "more than 256 labels share one representative");
     const int log_r = plan->n_base > 5 ? plan->n_base - 5 : 0;
     double2* sbuf[2] = {reinterpret_cast<double2*>(d_work), reinterpret_cast<double2*>((char*)d_work + sb)};
     double* part = reinterpret_cast<double*>((char*)d_work + 2 * sb);
@@ -1728,25 +1758,6 @@ extern "C" int qck_sim_tree(qck_handle* h, const qck_sim_tree_plan* plan, int64_
             *T, first, l, items, sbuf[(l + 1) & 1], sbuf[l & 1], part);
         QCK_CHECK_LAUNCH(h);
     }
-    int n_fork_max = 0;
-    long long n_rep_labels = 1, n_eq_max = 1;
-    for (int l = 0; l < plan->n_levels; ++l) {
-        const qck_tree_level& L = plan->level[l];
-        if (L.kind == QCK_TREE_MMEAS) continue;
-        n_fork_max += L.kind == QCK_TREE_SLOT;
-        int reps = 0, biggest = 1;
-        for (int v = 0; v < 8; ++v) {
-            if (L.first_choice[v] < 0) continue;
-            ++reps;
-            int cls = 0;
-            for (int d = 0; d < plan->radix[L.digit]; ++d) cls += (int)((L.canon >> (4 * d)) & 15u) == v;
-            if (cls > biggest) biggest = cls;
-        }
-        n_rep_labels *= reps;
-        n_eq_max *= biggest;
-    }
-    if (n_fork_max > 8) QCK_FAIL(h, QCK_ERR_UNSUPPORTED, "more than 8 measuring slots whose qubit lives on");
-    if (n_eq_max > 256) QCK_FAIL(h, QCK_ERR_UNSUPPORTED, "more than 256 labels share one representative");
     unsigned long long cg = ((unsigned long long)n_rep_labels + QCK_TREE_COMBINE_WARPS - 1) / QCK_TREE_COMBINE_WARPS;
     if (cg > (unsigned long long)h->sm_count * 8) cg = (unsigned long long)h->sm_count * 8;
     sim_tree_combine_kernel<<<(unsigned)cg, 32 * QCK_TREE_COMBINE_WARPS, 0, st>>>(

@@ -142,7 +142,9 @@ typedef struct {
     /* output row: bit j of the row index <- state bit out_pos[j] (-1: the bit is
      * never set, entries with it set are 0).  Bits in sum_mask are summed out,
      * those also in sign_mask with weight (-1)^bit (signed fold of the config
-     * bits, SURVEY.md A.3). */
+     * bits, SURVEY.md A.3).  A QCK_SWEEP_WARP plan must keep sign_mask inside sum_mask
+     * (that kernel signs every set bit, the others only summed ones) and make every outcome
+     * bit an out_pos bit or a sum_mask bit (every leaf is added): else QCK_ERR_INVALID_ARG. */
     int32_t n_out_bits;
     int32_t out_pos[QCK_MAX_OUT_BITS];
     uint64_t sum_mask;
