@@ -91,6 +91,16 @@ class QckDmPlan(C.Structure):
                 ("qcol", C.c_int32 * DM_MAX_QUBITS), ("n_digits", C.c_int32), ("radix", C.c_int32 * MAX_DIGITS)]
 
 
+TRAJ_OP_INTS, TRAJ_SMEM_MAX_QUBITS = 8, 13
+
+
+class QckTrajPlan(C.Structure):
+    _fields_ = [("n_qubits", C.c_int32), ("n_ops", C.c_int32), ("d_ops", C.c_void_p), ("d_vars", C.c_void_p),
+                ("d_mats", C.c_void_p), ("d_labels", C.c_void_p), ("n_labels", C.c_int64), ("d_ro", C.c_void_p),
+                ("n_cols", C.c_int32), ("fold_bits", C.c_int32), ("n_digits", C.c_int32), ("term_uidx", C.c_int32),
+                ("ro_cols", C.c_uint32), ("qcol", C.c_int32 * DM_MAX_QUBITS)]
+
+
 class QckStats(C.Structure):
     _fields_ = [("sum", C.c_double), ("min", C.c_double), ("sum_sqrt", C.c_double), ("nnz", C.c_double)]
 
@@ -164,6 +174,9 @@ _PROTOTYPES = {
                                   C.c_void_p]),
     "qck_sim_density": (C.c_int, [C.c_void_p, C.POINTER(QckDmPlan), C.c_int64, C.c_int64, C.c_void_p, C.c_int64,
                                   C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "qck_sim_trajectories": (C.c_int, [C.c_void_p, C.POINTER(QckTrajPlan), C.c_int64, C.c_int64, C.c_int64,
+                                       C.c_uint64, C.c_uint32, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
+                                       C.c_size_t, C.c_void_p]),
     "qck_stats_dense": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.c_void_p, C.c_void_p]),
     "qck_hellinger": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
     "qck_npd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.POINTER(C.c_double),

@@ -22,6 +22,12 @@ backend bound to fragments makes ``run_virtual_circuit(virt, shots)`` sample eve
 distribution, or with ``sampling=True`` a multinomial of it - what a noisy Aer backend returns.  Bound to fragments,
 it gives every fragment instance its noisy table.  ``noise_model=None`` is the noiseless state-vector path.
 
+``method`` chooses how a noise model is simulated, as Aer's ``method`` does: ``"density_matrix"`` (the default) is
+the density path above; ``"statevector"`` needs ``sampling=True`` and draws every shot as one stochastic state-vector
+trajectory (``trajectory.py``, ``qck_sim_trajectories``): ``shots · 2^n`` work per circuit instead of ``4^n``, so
+circuits and fragments up to 20 qubits run where a density matrix does not fit.  Without a noise model ``method``
+changes nothing.  The choice is the user's: switching methods changes the counts a seeded run draws.
+
 ``run_virtual_circuit`` recognises this class and bypasses circuit objects,
 strings and dicts entirely (``VirtualCircuit.simulate_fragments``).
 """
@@ -59,11 +65,24 @@ class B200Job:
 class B200Backend:
     name = "b200_statevector"
 
-    def __init__(self, device=None, sampling: bool = False, seed: int | None = None, noise_model=None) -> None:
+    METHODS = ("density_matrix", "statevector")
+
+    def __init__(self, device=None, sampling: bool = False, seed: int | None = None, noise_model=None,
+                 method: str = "density_matrix") -> None:
+        if method not in self.METHODS:
+            raise ValueError(f"method {method!r}: one of {self.METHODS}")
+        if method == "statevector" and noise_model is not None and not sampling:
+            raise ValueError("method='statevector' under a noise model samples trajectories: it needs sampling=True")
         self._device = device
         self.sampling = bool(sampling)
         self.seed = seed
         self.noise_model = noise_model
+        self.method = method
+
+    @property
+    def trajectories(self) -> bool:
+        """Noisy shots are drawn as state-vector trajectories (``method="statevector"`` with a noise model)."""
+        return self.method == "statevector" and self.noise_model is not None and self.sampling
 
     def next_seed(self) -> int:
         """The Philox key of one call: ``seed``, or a fresh one when it is None."""
@@ -77,8 +96,8 @@ class B200Backend:
             off += len(reg)
         return " ".join(reversed(parts))
 
-    def _row(self, circuit: QuantumCircuit):
-        """-> (program, device row [1, 2^m] of the exact outcome distribution), or (program, None)."""
+    def _flat(self, circuit: QuantumCircuit):
+        """-> (the circuit on one register, that register, device, handle)."""
         device = self._device if self._device is not None else default_device()
         handle = _lib.get_handle(getattr(device, "index", None) or 0)
         whole = QuantumRegister(circuit.num_qubits, "all")
@@ -86,6 +105,11 @@ class B200Backend:
         flat = QuantumCircuit(whole, *circuit.cregs)
         for ins in circuit.data:
             flat.append(ins.operation, [remap[q] for q in ins.qubits], ins.clbits)
+        return flat, whole, device, handle
+
+    def _row(self, circuit: QuantumCircuit):
+        """-> (program, device row [1, 2^m] of the exact outcome distribution), or (program, None)."""
+        flat, whole, device, handle = self._flat(circuit)
         if self.noise_model is not None:
             from .density import DensityExecutor, DensityProgram
             prog = DensityProgram(flat, whole, circuit.num_clbits, self.noise_model)
@@ -118,6 +142,8 @@ class B200Backend:
         """``shots`` samples of one circuit's outcome (key bit i = clbit i) -> integer counts.  Only the sorted
         shot list comes back to the host."""
         import torch
+        if self.trajectories:
+            return self._trajectory_counts(circuit, shots, seed, stream_id)
         prog, row, handle = self._row(circuit)
         if row is None:
             return {}
@@ -129,6 +155,21 @@ class B200Backend:
         host = torch.cat([shot_list[0], status]).cpu().numpy()    # one read-back: the shots and the status word
         _sampling.raise_for_status(int(host[-1]))
         cols, counts = np.unique(host[:-1], return_counts=True)
+        keys = self._keys(cols, prog.out_clbits)
+        return {int(k): int(n) for k, n in zip(keys.tolist(), counts.tolist())}
+
+    def _trajectory_counts(self, circuit: QuantumCircuit, shots: int, seed: int, stream_id: int) -> dict[int, int]:
+        """``sample_counts`` by trajectories: the shot list is the only read-back."""
+        import torch
+        from .trajectory import TrajectoryExecutor, TrajectoryProgram
+        flat, whole, device, handle = self._flat(circuit)
+        prog = TrajectoryProgram(flat, whole, circuit.num_clbits, self.noise_model)
+        if not prog.measures_anything:
+            return {}
+        shot_list = torch.empty((1, int(shots)), dtype=torch.int64, device=device)
+        TrajectoryExecutor(prog, device).sample(handle, shots, seed, stream_id, shot_list=shot_list,
+                                                stream=torch.cuda.current_stream(device).cuda_stream)
+        cols, counts = np.unique(shot_list[0].cpu().numpy(), return_counts=True)
         keys = self._keys(cols, prog.out_clbits)
         return {int(k): int(n) for k, n in zip(keys.tolist(), counts.tolist())}
 

@@ -129,6 +129,29 @@ __host__ __device__ __forceinline__ uint64_t soft_pdep(uint64_t x, uint64_t mask
     return out;
 }
 
+// ---- Philox4x32-10 and its uniforms (sample.cu, trajectory.cu; tests/sampling_reference.py restates both)
+__device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0,
+                                              uint32_t k1, uint32_t out[4]) {
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
+        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
+        c0 = hi1 ^ c1 ^ k0;
+        c1 = lo1;
+        c2 = hi0 ^ c3 ^ k1;
+        c3 = lo0;
+        k0 += 0x9E3779B9u;
+        k1 += 0xBB67AE85u;
+    }
+    out[0] = c0, out[1] = c1, out[2] = c2, out[3] = c3;
+}
+
+// x = lo | hi << 32 -> ((x >> 11) | 1) * 2^-53: an exact double in [2^-53, 1 - 2^-53]
+__device__ __forceinline__ double qck_uniform(uint32_t lo, uint32_t hi) {
+    const unsigned long long x = (unsigned long long)lo | ((unsigned long long)hi << 32);
+    return (double)((x >> 11) | 1ull) * 0x1p-53;
+}
+
 // ---- block reductions ------------------------------------------------------------------
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll

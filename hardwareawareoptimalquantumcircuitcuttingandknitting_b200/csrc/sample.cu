@@ -21,25 +21,7 @@ int qck_ensure_scratch(qck_handle* h, size_t bytes, void** out);  // api.cu
 #define SP_ST_ENTRY 1ull       // an entry is negative, NaN or infinite
 #define SP_ST_TOTAL 2ull       // a row total is not > 0 or not finite
 
-// ---------------------------------------------------------------------------------------------------- Philox4x32-10
-__device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0,
-                                              uint32_t k1, uint32_t out[4]) {
-#pragma unroll
-    for (int r = 0; r < 10; ++r) {
-        const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
-        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
-        c0 = hi1 ^ c1 ^ k0;
-        c1 = lo1;
-        c2 = hi0 ^ c3 ^ k1;
-        c3 = lo0;
-        k0 += 0x9E3779B9u;
-        k1 += 0xBB67AE85u;
-    }
-    out[0] = c0, out[1] = c1, out[2] = c2, out[3] = c3;
-}
-
-// The uniforms of one node's draw: Philox call t gives two, (w0, w1) then (w2, w3); x = lo | hi << 32 becomes
-// ((x >> 11) | 1) * 2^-53, an exact double in [2^-53, 1 - 2^-53].
+// The uniforms of one node's draw: Philox call t gives two, (w0, w1) then (w2, w3) (qck_uniform).
 struct NodeRng {
     uint32_t c0, c1, c2, c3, k0, k1;
     uint32_t w[4];
@@ -52,8 +34,7 @@ struct NodeRng {
         const int half = used & 1;
         if (!half) philox4x32_10(c0, c1, c2, c3 + (uint32_t)(used >> 1), k0, k1, w);
         ++used;
-        const unsigned long long x = (unsigned long long)w[2 * half] | ((unsigned long long)w[2 * half + 1] << 32);
-        return (double)((x >> 11) | 1ull) * 0x1p-53;
+        return qck_uniform(w[2 * half], w[2 * half + 1]);
     }
 };
 

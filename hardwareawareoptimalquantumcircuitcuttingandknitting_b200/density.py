@@ -48,21 +48,18 @@ def _unitary_superop(u: np.ndarray) -> np.ndarray:
     return np.kron(np.conj(u), u)
 
 
-class DensityProgram:
-    """One fragment lowered for ``qck_sim_density``.  Row layout, ``out_clbits``, ``radix`` and ``num_labels`` are
-    those of the fragment's ``FragmentProgram``."""
+class NoisyLowering:
+    """One fragment and a noise model lowered into per-op channels (superoperators), branch bits, row columns and
+    readout tables: what ``DensityProgram`` schedules into sweeps and ``trajectory.TrajectoryProgram`` unravels into
+    Kraus operators.  Row layout, ``out_clbits``, ``radix`` and ``num_labels`` are those of the fragment's
+    ``FragmentProgram``."""
 
-    def __init__(self, frag_circuit: QuantumCircuit, fragment: QuantumRegister, num_clbits: int, noise_model,
-                 tile_bits: int = TILE_BITS) -> None:
+    def __init__(self, frag_circuit: QuantumCircuit, fragment: QuantumRegister, num_clbits: int, noise_model) -> None:
         self.fragment = fragment
-        self.n_qubits = n = len(fragment)
-        if n > MAX_QUBITS:
-            raise MemoryError(f"a density matrix of {n} qubits does not fit any device")
+        self.n_qubits = len(fragment)
         self.num_clbits = num_clbits
         self.noise_model = noise_model
-        self.tile_bits = tile_bits
         self._lower(frag_circuit)
-        self._schedule()
 
     # ------------------------------------------------------------------ lowering
     def _gate_superop(self, name: str, params, qubits, matrix=None) -> np.ndarray:
@@ -204,6 +201,110 @@ class DensityProgram:
         self._mid_branches, self._slot_branch, self._term_slot = mid_branches, slot_branch, term_slot
         self._items_all = None
 
+    # ------------------------------------------------------------------ labels and items
+    def label_digits(self, labels: np.ndarray) -> np.ndarray:
+        if not self.radix:
+            return np.zeros((len(labels), 0), dtype=np.int64)
+        return np.stack(np.unravel_index(np.asarray(labels, dtype=np.int64), self.radix), axis=1)
+
+    def canonical_labels(self) -> np.ndarray:
+        """int32 [num_labels]: the smallest label whose instance is identical to this one, from the NOISY variant
+        data (two variants with one matrix but different op names can carry different noise)."""
+        cached = getattr(self, "_canon", None)
+        if cached is not None:
+            return cached
+        labels = np.arange(self.num_labels, dtype=np.int64)
+        if self.radix:
+            maps = []
+            for d, r in enumerate(self.radix):
+                first, m = {}, np.zeros(r, dtype=np.int64)
+                for v in range(r):
+                    m[v] = first.setdefault(tuple(s[v] for s in self.slot_keys[d]), v)
+                maps.append(m)
+            digits = self.label_digits(labels)
+            labels = np.ravel_multi_index(tuple(maps[d][digits[:, d]] for d in range(len(self.radix))), self.radix)
+        self._canon = labels.astype(np.int32)
+        return self._canon
+
+    def label_qmask(self, digits: np.ndarray) -> np.ndarray:
+        """int64 [n]: the qubits whose terminal bit a label's row records (a terminal slot's qubit only when the
+        label's variant measures)."""
+        qmask = np.zeros(len(digits), dtype=np.int64)
+        for q in range(self.n_qubits):
+            if self.qcol[q] < 0:
+                continue
+            if q in self._term_slot:
+                d, meas = self._term_slot[q]
+                qmask |= np.asarray(meas, dtype=np.int64)[digits[:, d]] << q
+            else:
+                qmask |= 1 << q
+        return qmask
+
+    def items(self, labels: np.ndarray):
+        """-> (items [n] of _ITEM sorted by label, item_begin int64 [num_labels + 1] counting only ``labels``)."""
+        labels = np.asarray(labels, dtype=np.int64)
+        digits = self.label_digits(labels)
+        active = np.zeros((len(labels), self.n_branch), dtype=bool)
+        for b in self._mid_branches:
+            active[:, b] = True
+        for d, b, meas in self._slot_branch:
+            active[:, b] = np.asarray(meas)[digits[:, d]]
+        qmask = self.label_qmask(digits)
+        packed = np.zeros(len(labels), dtype=np.uint64)
+        for d in range(len(self.radix)):
+            packed |= digits[:, d].astype(np.uint64) << np.uint64(4 * d)
+        n_items = 1 << active.sum(axis=1)
+        total = int(n_items.sum())
+        out = np.zeros(total, dtype=_ITEM)
+        owner = np.repeat(np.arange(len(labels)), n_items)
+        first = np.concatenate([[0], np.cumsum(n_items)[:-1]]).astype(np.int64)
+        rank = np.arange(total, dtype=np.int64) - first[owner]      # branch word over the ACTIVE bits
+        branch = np.zeros(total, dtype=np.int64)
+        col_base = np.zeros(total, dtype=np.int64)
+        j = np.zeros(total, dtype=np.int64)                          # next bit of rank to consume
+        for b in range(self.n_branch):
+            on = active[owner, b]
+            bit = np.where(on, (rank >> j) & 1, 0)
+            branch |= bit << b
+            col_base |= bit << self.branch_col[b]
+            j += on
+        out["digits"] = packed[owner]
+        out["label"] = labels[owner]
+        out["branch"] = branch
+        out["col_base"] = col_base
+        out["qmask"] = qmask[owner]
+        begin = np.zeros(self.num_labels + 1, dtype=np.int64)
+        np.add.at(begin, labels + 1, n_items)
+        return out, np.cumsum(begin)
+
+    def ro_masks(self) -> np.ndarray:
+        """uint32 [num_labels]: the row columns whose readout error applies to a label (a configuration bit only
+        when the label's variant measures)."""
+        labels = np.arange(self.num_labels, dtype=np.int64)
+        digits = self.label_digits(labels)
+        mask = np.zeros(self.num_labels, dtype=np.int64)
+        for j in range(self.row_bits):
+            if self._ro_has[j, 0]:
+                mask |= 1 << j
+        for d in range(len(self.radix)):
+            mask |= self._ro_has[self.row_bits + d, :][digits[:, d]].astype(np.int64) << (self.row_bits + d)
+        return mask.astype(np.uint32)
+
+    def row_len(self, fold: bool = True) -> int:
+        return 1 << (self.row_bits + (0 if fold else len(self.radix)))
+
+
+class DensityProgram(NoisyLowering):
+    """One fragment lowered for ``qck_sim_density``: the shared lowering, scheduled into sweeps."""
+
+    def __init__(self, frag_circuit: QuantumCircuit, fragment: QuantumRegister, num_clbits: int, noise_model,
+                 tile_bits: int = TILE_BITS) -> None:
+        if len(fragment) > MAX_QUBITS:
+            raise MemoryError(f"a density matrix of {len(fragment)} qubits does not fit any device")
+        self.tile_bits = tile_bits
+        super().__init__(frag_circuit, fragment, num_clbits, noise_model)
+        self._schedule()
+
     # ------------------------------------------------------------------ sweeps
     def _schedule(self) -> None:
         n2 = 2 * self.n_qubits
@@ -258,94 +359,9 @@ class DensityProgram:
             self.sweeps.append((pos, first, len(recs)))
         self.op_records = np.asarray(recs, dtype=np.int32).reshape(-1, 12)
 
-    # ------------------------------------------------------------------ labels and items
-    def label_digits(self, labels: np.ndarray) -> np.ndarray:
-        if not self.radix:
-            return np.zeros((len(labels), 0), dtype=np.int64)
-        return np.stack(np.unravel_index(np.asarray(labels, dtype=np.int64), self.radix), axis=1)
-
-    def canonical_labels(self) -> np.ndarray:
-        """int32 [num_labels]: the smallest label whose instance is identical to this one, from the NOISY variant
-        data (two variants with one matrix but different op names can carry different noise)."""
-        cached = getattr(self, "_canon", None)
-        if cached is not None:
-            return cached
-        labels = np.arange(self.num_labels, dtype=np.int64)
-        if self.radix:
-            maps = []
-            for d, r in enumerate(self.radix):
-                first, m = {}, np.zeros(r, dtype=np.int64)
-                for v in range(r):
-                    m[v] = first.setdefault(tuple(s[v] for s in self.slot_keys[d]), v)
-                maps.append(m)
-            digits = self.label_digits(labels)
-            labels = np.ravel_multi_index(tuple(maps[d][digits[:, d]] for d in range(len(self.radix))), self.radix)
-        self._canon = labels.astype(np.int32)
-        return self._canon
-
-    def items(self, labels: np.ndarray):
-        """-> (items [n] of _ITEM sorted by label, item_begin int64 [num_labels + 1] counting only ``labels``)."""
-        labels = np.asarray(labels, dtype=np.int64)
-        digits = self.label_digits(labels)
-        active = np.zeros((len(labels), self.n_branch), dtype=bool)
-        for b in self._mid_branches:
-            active[:, b] = True
-        for d, b, meas in self._slot_branch:
-            active[:, b] = np.asarray(meas)[digits[:, d]]
-        qmask = np.zeros(len(labels), dtype=np.int64)
-        for q in range(self.n_qubits):
-            if self.qcol[q] < 0:
-                continue
-            if q in self._term_slot:
-                d, meas = self._term_slot[q]
-                qmask |= np.asarray(meas, dtype=np.int64)[digits[:, d]] << q
-            else:
-                qmask |= 1 << q
-        packed = np.zeros(len(labels), dtype=np.uint64)
-        for d in range(len(self.radix)):
-            packed |= digits[:, d].astype(np.uint64) << np.uint64(4 * d)
-        n_items = 1 << active.sum(axis=1)
-        total = int(n_items.sum())
-        out = np.zeros(total, dtype=_ITEM)
-        owner = np.repeat(np.arange(len(labels)), n_items)
-        first = np.concatenate([[0], np.cumsum(n_items)[:-1]]).astype(np.int64)
-        rank = np.arange(total, dtype=np.int64) - first[owner]      # branch word over the ACTIVE bits
-        branch = np.zeros(total, dtype=np.int64)
-        col_base = np.zeros(total, dtype=np.int64)
-        j = np.zeros(total, dtype=np.int64)                          # next bit of rank to consume
-        for b in range(self.n_branch):
-            on = active[owner, b]
-            bit = np.where(on, (rank >> j) & 1, 0)
-            branch |= bit << b
-            col_base |= bit << self.branch_col[b]
-            j += on
-        out["digits"] = packed[owner]
-        out["label"] = labels[owner]
-        out["branch"] = branch
-        out["col_base"] = col_base
-        out["qmask"] = qmask[owner]
-        begin = np.zeros(self.num_labels + 1, dtype=np.int64)
-        np.add.at(begin, labels + 1, n_items)
-        return out, np.cumsum(begin)
-
-    def ro_masks(self) -> np.ndarray:
-        """uint32 [num_labels]: the row columns whose readout error applies to a label (a configuration bit only
-        when the label's variant measures)."""
-        labels = np.arange(self.num_labels, dtype=np.int64)
-        digits = self.label_digits(labels)
-        mask = np.zeros(self.num_labels, dtype=np.int64)
-        for j in range(self.row_bits):
-            if self._ro_has[j, 0]:
-                mask |= 1 << j
-        for d in range(len(self.radix)):
-            mask |= self._ro_has[self.row_bits + d, :][digits[:, d]].astype(np.int64) << (self.row_bits + d)
-        return mask.astype(np.uint32)
-
-    def row_len(self, fold: bool = True) -> int:
-        return 1 << (self.row_bits + (0 if fold else len(self.radix)))
-
     def rho_bytes(self) -> int:
         return 16 << (2 * self.n_qubits)
+
 
 
 class DensityExecutor:

@@ -375,9 +375,12 @@ def run_virtual_circuit(virt: VirtualCircuit, shots: int = 20000) -> tuple[dict[
             if virt.program(frag).measures_anything:
                 if backend.sampling:
                     status = new_status(torch, device) if status is None else status
-                    unfolded = virt.executor(frag, device, False).run(handle)
-                    tables[frag] = virt.sample_table(handle, frag, unfolded, fold, shots, status,
-                                                     stream=torch.cuda.current_stream(device).cuda_stream)
+                    stream = torch.cuda.current_stream(device).cuda_stream
+                    if backend.trajectories:
+                        tables[frag] = virt.sample_trajectories(handle, frag, device, fold, shots, stream=stream)
+                    else:
+                        unfolded = virt.executor(frag, device, False).run(handle)
+                        tables[frag] = virt.sample_table(handle, frag, unfolded, fold, shots, status, stream=stream)
                 else:
                     tables[frag] = virt.executor(frag, device, fold).run(handle)
             continue

@@ -224,8 +224,9 @@ class VirtualCircuit:
         return self._programs[fragment]
 
     def executor(self, fragment: Fragment, device, fold: bool = True) -> FragmentExecutor:
-        """The fragment's executor: its density-matrix program (``density.py``) when the fragment is bound to a
-        ``B200Backend(noise_model=...)``, its state-vector program otherwise.  Both fill the same table layout."""
+        """The fragment's executor of exact tables: its density-matrix program (``density.py``) when the fragment is
+        bound to a ``B200Backend(noise_model=...)``, whatever its ``method``, its state-vector program otherwise.  Both
+        fill the same table layout.  Sampled tables of a trajectory backend come from ``trajectory_executor``."""
         model = self.noise_model(fragment)
         # keyed on the model and its revision too: a backend's model can be swapped or extended between runs
         key = (fragment, str(device), fold, model, None if model is None else model.revision)
@@ -238,10 +239,26 @@ class VirtualCircuit:
                 self._executors[key] = FragmentExecutor(self.program(fragment), device, fold)
         return self._executors[key]
 
+    def trajectory_executor(self, fragment: Fragment, device):
+        """The fragment's trajectory executor (``trajectory.py``): one device image for folded and unfolded tables,
+        cached with the executors (same key rules, so ``set_backend`` drops it)."""
+        from .trajectory import TrajectoryExecutor, TrajectoryProgram
+        model = self.noise_model(fragment)
+        key = (fragment, str(device), "trajectory", model, model.revision)
+        if key not in self._executors:
+            prog = TrajectoryProgram(self._frag_circs[fragment], fragment, self.num_clbits, model)
+            self._executors[key] = TrajectoryExecutor(prog, device)
+        return self._executors[key]
+
     def noise_model(self, fragment: Fragment):
         """The noise model of the ``B200Backend`` the fragment is bound to (None: noiseless or a foreign backend)."""
         return getattr(self._frag_to_backend[fragment], "noise_model", None) if isinstance(
             self._frag_to_backend[fragment], _b200_backend_type()) else None
+
+    def trajectory_fragment(self, fragment: Fragment) -> bool:
+        """The fragment's backend draws noisy shots as state-vector trajectories (``B200Backend.trajectories``)."""
+        be = self._frag_to_backend[fragment]
+        return isinstance(be, _b200_backend_type()) and be.trajectories
 
     def noisy_fragments(self) -> list[Fragment]:
         """Active fragments bound to a ``B200Backend(noise_model=...)``."""
@@ -340,19 +357,24 @@ class VirtualCircuit:
         ``shots``: every fragment whose backend samples (``B200Backend(sampling=True)``) is simulated unfolded and
         each instance's row is replaced by a multinomial sample of ``shots`` divided by ``shots``, in the layout
         ``fold`` asks for (``qck_rows_sample``; stream id = the fragment's index in ``fragment_circuits``, row label
-        = the fragment label, so label ranges draw the rows of the full run).  Fragments on exact backends are
-        unchanged.  The status word of the sampler is left in ``self.sample_status`` (device int64, 0 = the tables
+        = the fragment label, so label ranges draw the rows of the full run).  A fragment on a
+        ``B200Backend(noise_model=..., sampling=True, method="statevector")`` draws its shots as trajectories
+        (``qck_sim_trajectories``, same seed, stream id and row labels) without an exact table.  Fragments on exact
+        backends are unchanged.  The status word of the sampler is left in ``self.sample_status`` (device int64, 0 = the tables
         were valid); ``check_sample_status()`` reads it.  Observables take these tables unchanged
         (``expectation_values(virt, z_masks, tables=virt.simulate_fragments(dev, shots=N))``)."""
         device = default_device() if device is None else device
         sampled = set(self.sampling_fragments()) if shots is not None else set()
         if sampled:
             return self._simulate_sampled(device, label_range, fold, out, int(shots), sampled)
+        return self._simulate_exact(device, label_range, fold, out, self.active_fragments())
+
+    def _simulate_exact(self, device, label_range, fold, out, frags) -> dict:
+        """The exact tables of ``frags`` (``simulate_fragments`` without ``shots``)."""
         handle = _lib.get_handle(getattr(device, "index", None) or 0)
         import torch
         stream = torch.cuda.current_stream(device).cuda_stream
         tables, runs = {}, []
-        frags = self.active_fragments()
         # the fragments are independent jobs (run.py:36-43): inside a region their launches overlap on the GPU
         overlap = len(frags) > 1
         # Everything that enqueues work on the caller's stream - the H2D copy of a program, the zero-fill of a
@@ -386,12 +408,20 @@ class VirtualCircuit:
     def _simulate_sampled(self, device, label_range, fold, out, shots, sampled) -> dict:
         import torch
         from . import sampling as _sampling
-        exact = self.simulate_fragments(device, label_range, fold=False, shots=None)
+        # trajectory fragments go straight to their sampled tables; the others are simulated exactly, then sampled
+        traj = {f for f in sampled if self.trajectory_fragment(f)}
+        exact = self._simulate_exact(device, label_range, False, None,
+                                     [f for f in self.active_fragments() if f not in traj])
         handle = _lib.get_handle(getattr(device, "index", None) or 0)
         stream = torch.cuda.current_stream(device).cuda_stream
         self.sample_status = _sampling.new_status(torch, device)
         tables = {}
-        for frag, table in exact.items():
+        for frag in self.active_fragments():
+            if frag in traj:
+                tables[frag] = self.sample_trajectories(handle, frag, device, fold, shots, label_range,
+                                                        out[frag] if out is not None else None, stream)
+                continue
+            table = exact[frag]
             if frag not in sampled:
                 if fold:        # an exact fragment keeps its folded table
                     table = self.executor(frag, device, True).run(
@@ -422,6 +452,23 @@ class VirtualCircuit:
         _sampling.rows_sample(handle, unfolded, prog.row_bits + len(prog.radix), shots, seed, stream_id, status,
                               l0, l1, out=out, fold_bits=f, stream=stream)
         return out
+
+    def sample_trajectories(self, handle, frag: Fragment, device, fold: bool, shots: int,
+                            label_range: tuple[int, int] | None = None, out=None, stream: int = 0):
+        """Sampled table of one trajectory fragment (``qck_sim_trajectories``), with the seed, stream id and row
+        labels of ``sample_table``."""
+        import torch
+        ex = self.trajectory_executor(frag, device)
+        prog = ex.program
+        seed = self._frag_to_backend[frag].next_seed()
+        stream_id = list(self._frag_circs).index(frag)
+        l0, l1 = (0, prog.num_labels)
+        if label_range is not None and self._vgate_instrs:
+            l0, l1 = self.fragment_label_range(frag, *label_range)
+        if out is None:
+            alloc = torch.zeros if (l0, l1) != (0, prog.num_labels) else torch.empty
+            out = alloc((prog.num_labels, prog.row_len(fold)), dtype=torch.float64, device=device)
+        return ex.sample(handle, shots, seed, stream_id, (l0, l1), out=out, fold=fold, stream=stream)
 
     def check_sample_status(self) -> None:
         """Raises ValueError when the last sampled ``simulate_fragments`` met an invalid table (synchronises)."""

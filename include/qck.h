@@ -499,6 +499,63 @@ QCK_API int qck_sim_density(qck_handle* h, const qck_dm_plan* plan, int64_t labe
                             double* d_out, int64_t out_row_stride, double* d_rows, void* d_work, size_t work_bytes,
                             qck_stream stream);
 
+/* ------------------------------------------------------------------ noisy shots by quantum trajectories
+ * Replaces: backend.run(instantiations, shots) on AerSimulator(method="statevector", noise_model=nm) (run.py:42):
+ * every shot of every instance is one stochastic state-vector trajectory (trajectory.py lowers a fragment and a
+ * noise model into this plan, from the same per-op channels as qck_dm_plan).  Costs shots * 2^n per instance
+ * instead of 4^n.
+ *
+ * Op record (int32[8]): {nq, q0, q1, sel_digit, col, uidx, var_off, 0}.  The op acts on qubits q0 (local index bit
+ * 0) and q1 (bit 1, nq = 2).  Its variant is v = the label's digit sel_digit (0 when < 0); d_vars[var_off + v] =
+ * {n_kraus, mat_off}: n_kraus operators K_k (d x d, d = 2^nq, row-major [out][in]), each followed by
+ * M_k = K_k^dag K_k, at d_mats + mat_off (complex128).  n_kraus = 0: the identity.  uidx >= 0 when some variant
+ * has n_kraus >= 2; col >= 0 when the op records a bit (a measurement) in that row column.
+ * Label record (16 bytes): {uint64 digits (4 bits per digit), uint32 qmask, uint32 ro_mask}.
+ *
+ * Definition of trajectory (label, shot), label in [label_begin, label_end), shot in [0, shots):
+ *   - psi = |0...0> (2^n complex128, index bit q = qubit q), column c = 0;
+ *   - for every op with n_kraus >= 2 in its variant: rho = psi's reduced density matrix on the op's qubits,
+ *     p_k = max(0, Re Tr(M_k rho)), P_j = p_0 + ... + p_j (in k order); k = the smallest index with
+ *     u[uidx] * P_{n-1} < P_k; psi <- K_k psi / sqrt(p_k); with col >= 0, c |= k << col.
+ *     n_kraus = 1: psi <- K_0 psi.  n_kraus = 0: nothing;
+ *   - terminal sample: i = the smallest index with u[term_uidx] * S < sum_{j <= i} |psi_j|^2 in index order
+ *     (S = the whole sum); c |= bit q of i << qcol[q] for every q in the label's qmask;
+ *   - readout: for each column j in the label's ro_mask, in ascending order, with m = bit j of c and
+ *     R = d_ro[j][v] (R[o][i] = p(recorded o | measured i) at 2 o + i, v = the label's digit of a configuration
+ *     column j >= n_cols - n_digits, 0 for a clbit column): bit j of c <- (u[term_uidx + 1 + r] < R[1][m]), r = the
+ *     number of ro_cols bits below j;
+ *   - u[j]: Philox4x32-10 keyed by (seed mod 2^32, seed >> 32) at counter (shot, label, stream_id, j >> 1), words
+ *     (w0, w1) for even j and (w2, w3) for odd j, converted as qck_rows_sample converts them.  So a trajectory's
+ *     draws depend on (seed, stream_id, label, shot) and the plan only, not on the label range, the launch or the
+ *     rank; the sums above are taken in an order that depends on n only (the same seed gives the same bits).
+ * Outputs (either or both):
+ *   d_out row `label` (absolute, stride out_row_stride): the counts of column c, folded with sign (-1)^bit over
+ *     the top fold_bits columns, as integers, divided by `shots` once: the layout and definition of
+ *     qck_rows_sample's d_out.  Padding past the row is not touched.
+ *   d_shot_list [label - label_begin][shot]: c of every trajectory, in shot order (unsorted).
+ * Regimes: n <= 13: one CTA per trajectory at a time with psi in shared memory; 14 <= n <= 20: persistent CTAs,
+ * each owning a psi slot of 16 << n bytes of d_work, grid-striding over the trajectories (no slot: QCK_ERR_NOMEM
+ * before anything is launched).  1 <= shots < 2^31, labels < 2^32.  No host synchronisation. */
+#define QCK_TRAJ_OP_INTS 8
+#define QCK_TRAJ_SMEM_MAX_QUBITS 13
+typedef struct {
+    int32_t n_qubits, n_ops;
+    const int32_t* d_ops;                /* [n_ops][QCK_TRAJ_OP_INTS] */
+    const int32_t* d_vars;               /* [][2] {n_kraus, mat_off} */
+    const double* d_mats;                /* complex128 pool */
+    const void* d_labels;                /* [n_labels] label records */
+    int64_t n_labels;
+    const double* d_ro;                  /* [n_cols][QCK_MAX_VARIANTS][4] */
+    int32_t n_cols, fold_bits, n_digits;
+    int32_t term_uidx;
+    uint32_t ro_cols;                    /* columns that have a readout error for some label */
+    int32_t qcol[QCK_DM_MAX_QUBITS];
+} qck_traj_plan;
+QCK_API int qck_sim_trajectories(qck_handle* h, const qck_traj_plan* plan, int64_t label_begin, int64_t label_end,
+                                 int64_t shots, uint64_t seed, uint32_t stream_id, double* d_out,
+                                 int64_t out_row_stride, int64_t* d_shot_list, void* d_work, size_t work_bytes,
+                                 qck_stream stream);
+
 /* ------------------------------------------------------------------ reductions
  * qck_stats_dense: sum / min / nnz of a dense vector (entries |v| <= acc count as absent).
  * qck_hellinger: result[0..2] = sum p, sum q, sum sqrt(p q) over max(.,0) entries; the
